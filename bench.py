@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the EWA-Jinc resampling hot path on B200, next to the reference's CPU path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 1..9] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 1..9] [--impl b200|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of `frames_per_step` distinct synthetic frames of the
 chosen BASELINE.json config (default: configs[1], 1080p YUV420P8 -> 2160p Jinc36Resize cplace=MPEG2).
@@ -21,6 +21,8 @@ Prints ONE JSON line (rank 0):
   cpu_baseline the UNMODIFIED reference (oracle/_ref) on this box's host cores, AVX2 and AVX-512 paths, one thread and
                all threads, on a bounded sample of the same workload, plus its filter construction time
 `--impl reference` times only that CPU reference and prints the same line shape with "impl": "reference".
+`--dump-outputs DIR` writes what the last kernel-only step computed as DIR/plane<i>.npy (float32, see dump_outputs); the
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 Under torchrun (N>1) every rank drives its own GPU with the same per-GPU batch (weak scaling; frames are
 independent, so there is no collective on the data path -- NCCL is used for the barrier and the max only).
 """
@@ -39,6 +41,7 @@ import time
 import numpy as np
 
 REPO = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (which may be read-only)
 sys.path.insert(0, REPO)
 sys.path.insert(0, os.path.join(REPO, "avisynth-jincresize_b200"))
 
@@ -241,12 +244,13 @@ def host_threads() -> int:
 OPT_NAMES = {2: "avx2", 3: "avx512"}
 
 
-def run_reference(cfg, steps: int, warmup: int, budget_s: float):
+def run_reference(cfg, steps: int, warmup: int, budget_s: float, exact_steps: bool = False):
     """Times the reference's own CPU implementation through its plugin API under the mini-host.  For each SIMD path the
     host CPU has (opt=2 AVX2 -- what the reference picks by default, src/JincResize.cpp:898 -- and opt=3 AVX-512, :897):
     filter construction (LUT + generate_coeff_table_c, :795-866), single-thread frames, then frame-parallel get_frame
     with one host thread per core (what AviSynth's Prefetch does for this MT_MULTI_INSTANCE filter).  `value` is the
-    faster path's all-thread figure.  Falls back to the scalar oracle port only if the prebuilt reference is absent."""
+    faster path's all-thread figure.  The step count is cut to fit `budget_s` unless exact_steps is set.  Falls back to the
+    scalar oracle port only if the prebuilt reference is absent."""
     fmt, w, h, tw, th = cfg["fmt"], cfg["w"], cfg["h"], cfg["tw"], cfg["th"]
     threads = host_threads()
     mpix = tw * th / 1e6
@@ -272,10 +276,11 @@ def run_reference(cfg, steps: int, warmup: int, budget_s: float):
             n1 = max(1, min(4, int(0.15 * per_opt / max(t1, 1e-6))))
             t1 = clip.pull(1, n1, 1) / n1
             est = t1 * F / max(1, min(threads, F))
-            n_steps = max(1, steps)
-            while n_steps > 1 and est * (n_steps + warmup) > 0.7 * per_opt:
-                n_steps -= 1
-            n_warm = warmup if est * (n_steps + warmup) <= 0.7 * per_opt else 0
+            n_steps, n_warm = max(1, steps), warmup
+            if not exact_steps:
+                while n_steps > 1 and est * (n_steps + warmup) > 0.7 * per_opt:
+                    n_steps -= 1
+                n_warm = warmup if est * (n_steps + warmup) <= 0.7 * per_opt else 0
             f0 = 8
             for _ in range(n_warm):
                 clip.pull(f0, F, threads)
@@ -310,12 +315,16 @@ def run_reference(cfg, steps: int, warmup: int, budget_s: float):
     t = oc.Table(pp[0], lut)
     construct_s = time.perf_counter() - t0
     rows = max(8, th // 64)
+    peak = float(fmt.peak) if fmt.bits < 32 else 0.0
+    for _ in range(warmup):
+        t.resize(planes[0], peak, rows=(th // 2, th // 2 + rows))
     t0 = time.perf_counter()
-    t.resize(planes[0], float(fmt.peak) if fmt.bits < 32 else 0.0, rows=(th // 2, th // 2 + rows))
+    for _ in range(steps):
+        t.resize(planes[0], peak, rows=(th // 2, th // 2 + rows))
     dt = time.perf_counter() - t0
-    value = (rows * tw / 1e6) / dt
+    value = steps * (rows * tw / 1e6) / dt
     return dict(value=value, unit=METRIC, cores=1, kind="port", sample=f"{rows} luma rows of one frame, scalar oracle port",
-                ms_per_step=dt * 1e3, steps=1, warmup=0, frames_per_step=rows / th, construct_ms=construct_s * 1e3)
+                ms_per_step=dt / steps * 1e3, steps=steps, warmup=warmup, frames_per_step=rows / th, construct_ms=construct_s * 1e3)
 
 
 def bind_to_gpu_numa(device_index: int):
@@ -450,6 +459,29 @@ def verify_against_oracle(cfg, captured):
         t.close()
     return {"ok": True, "against": "CPU oracle (oracle/jinc_oracle.c)", "frames_checked": len({c[0] for c in captured}),
             "rows_checked": rows_checked, "max_err": worst, "bar": "1e-5 relative" if fmt.bits == 32 else "1 LSB"}
+
+
+DUMP_BYTES = 60 << 20  # below 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, dst_by_frame, shapes):
+    """The output planes of the batch as out_dir/plane<i>.npy, float32, one array row per output row (row y of frame f
+    is batch row f * H + y).  When the batch holds more than DUMP_BYTES of float32 samples, every plane keeps the same
+    fraction of its batch rows, drawn by a fixed-seed generator and kept in batch order, so that runs with the same
+    arguments write the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    F = len(dst_by_frame)
+    frac = min(1.0, DUMP_BYTES / (4 * F * sum(h * w for _, (h, w) in shapes)))
+    rng = np.random.default_rng(0x4A494E43)
+    for i, (_, (H, W)) in enumerate(shapes):
+        n = F * H
+        rows = np.arange(n) if frac == 1.0 else np.sort(rng.choice(n, int(n * frac), replace=False))
+        out = np.empty((rows.size, W), np.float32)
+        for f in range(F):
+            sel = (rows >= f * H) & (rows < (f + 1) * H)
+            if sel.any():
+                out[sel] = dst_by_frame[f][i][:, :W].cpu().numpy()[rows[sel] - f * H]
+        np.save(os.path.join(out_dir, f"plane{i}.npy"), out)
 
 
 def copy_ceiling(D, host_src, host_dst, dev_src, dev_dst, inflight: int, steps: int):
@@ -603,6 +635,8 @@ def measure_config(D, args, cfg, config_id: int, steps: int, warmup: int, full: 
     dom_ms = [a.elapsed_time(b) for a, b in pairs]
     res = dict(F=F, fs_l=fs_l, fs_c=fs_c, infos=infos, ms_total=ms_total, dom_ms=dom_ms, gpu_launches=gpu_launches,
                construct_ms=sum(i.build_ms for i in infos), filter_create_ms=filter_create_s * 1e3, shapes=shapes)
+    if full and D.rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, dev_dst, shapes)
     captured = None
     if D.rank == 0 and args.parts == 3 and not args.no_verify:
         captured = capture_output_rows(cfg, [planes_np[0], planes_np[F - 1]], [dev_dst[0], dev_dst[F - 1]], shapes)
@@ -833,14 +867,21 @@ def main():
     ap.add_argument("--bands-config", type=int, default=4, choices=[4, 5], help="the 8K config whose single frame is cut into bands")
     ap.add_argument("--parts", type=int, default=3, choices=[1, 2, 3],
                     help="diagnosis only: 1 = interior tiles, 2 = border strips, 3 = both (the only valid bench setting)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the output planes of the last kernel-only step to DIR/plane<i>.npy (float32; a fixed-seed "
+                         "sample of whole rows when the batch exceeds 60 MiB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; it does not apply to --impl reference")
     cfg = CONFIGS[args.config]
     rank = int(os.environ.get("RANK", "0"))
 
     if args.impl == "reference":
         if rank != 0:
             return
-        r = run_reference(cfg, steps=args.steps, warmup=args.warmup, budget_s=150.0)
+        r = run_reference(cfg, steps=args.steps, warmup=args.warmup, budget_s=150.0, exact_steps=True)
         line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": "Mpixel/s", "n_gpus": args.gpus,
                 "steps": r["steps"], "warmup": r["warmup"], "ms_per_step": r["ms_per_step"], "higher_is_better": True,
                 "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",

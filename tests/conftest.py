@@ -18,8 +18,6 @@ def native_built():
     import subprocess
 
     subprocess.run(["make", "-s", "host"], cwd=REPO, check=True)
-    if os.path.isdir("/root/reference/src"):
-        subprocess.run(["make", "-s", "ref"], cwd=REPO, check=True)
     return True
 
 

@@ -13,7 +13,7 @@ from common import SMALL_CASES, make_planes, oracle_frame
 @pytest.fixture(scope="module")
 def ref(native_built, have_ref):
     if not have_ref:
-        pytest.skip("oracle/_ref not built (no /root/reference on this box)")
+        pytest.skip("oracle/_ref not built (`make ref` needs the reference sources)")
     from minihost import avs_host as ah
     from jinc_b200 import paths
 
