@@ -72,6 +72,8 @@ struct Up2xPlan {
     int sx0 = 0, sy0 = 0;     // window origin of cell (0,0), phase 0
     int ox1 = 0, oy1 = 0;     // extra origin offset of phase 1 on each axis (0 or 1)
     int wblock[2][2] = {{0, 0}, {0, 0}}; // [py][px] -> phase-block index
+    int taps = 0;      // tap-mask variant of integer planes (UpTaps<fs, taps>, jinc_up2x_taps.h); 0: every tap
+    int live_taps = 0; // taps per cell that variant multiplies
 };
 
 // Integer-ratio downscale interior (one phase).

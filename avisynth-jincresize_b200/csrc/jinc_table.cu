@@ -17,10 +17,12 @@
 #include <chrono>
 #include <climits>
 #include <cmath>
+#include <cstdlib>
 #include <cstring>
 #include <unordered_map>
 
 #include "jinc_internal.h"
+#include "jinc_up2x_taps.h"
 #include "jinc_weights.cuh"
 
 namespace {
@@ -569,6 +571,62 @@ void plan_fast_paths(jinc_table* t)
     }
 }
 
+// Tightest tap-mask variant of fs whose (ox1, oy1) is the table's and whose live columns contain every non-zero weight
+template <int FS, int M = 1>
+void pick_up2x_taps(const uint32_t (&nz)[2][2][FS], Up2xPlan& u)
+{
+    if constexpr (M < jinc_rs::UP_TAP_VARIANTS) {
+        using K = jinc_rs::UpTaps<FS, M>;
+        bool fits = K::OX1 == u.ox1 && K::OY1 == u.oy1;
+        int live = 0;
+        for (int py = 0; py < 2; ++py)
+            for (int px = 0; px < 2; ++px)
+                for (int ly = 0; ly < FS; ++ly) {
+                    fits = fits && (nz[py][px][ly] & ~K::cols(py, px, ly)) == 0;
+                    live += __builtin_popcount(K::cols(py, px, ly));
+                }
+        if (fits && live < u.live_taps) {
+            u.taps = M;
+            u.live_taps = live;
+        }
+        pick_up2x_taps<FS, M + 1>(nz, u);
+    }
+}
+
+template <int FS>
+void plan_up2x_taps_fs(const jinc_table* t, Up2xPlan& u)
+{
+    uint32_t nz[2][2][FS] = {}; // [py][px][ly]: bit lx set when that weight is not exactly zero
+    for (int py = 0; py < 2; ++py)
+        for (int px = 0; px < 2; ++px) {
+            const float* blk = t->h_weights.data() + (size_t)u.wblock[py][px] * FS * FS;
+            for (int ly = 0; ly < FS; ++ly)
+                for (int lx = 0; lx < FS; ++lx)
+                    nz[py][px][ly] |= (blk[ly * FS + lx] != 0.f ? 1u : 0u) << lx;
+        }
+    pick_up2x_taps<FS>(nz, u);
+}
+
+// The exact-2x kernel of integer planes skips the taps a compiled mask marks as zero (jinc_up2x_taps.h).  A mask is
+// used only when every weight it skips is exactly zero in this table, so the choice can cost speed but never change a
+// result.  JINCRESIZE_B200_UP2X_ZERO_TAPS=0 keeps every tap (the byte-identity reference of the tests).
+void plan_up2x_taps(jinc_table* t)
+{
+    Up2xPlan& u = t->up2x;
+    const int fs = t->sc.fs;
+    u.taps = 0;
+    u.live_taps = 4 * fs * fs;
+    if (t->fast_path != JINC_PATH_UP2X || t->h_weights.empty())
+        return;
+    const char* off = getenv("JINCRESIZE_B200_UP2X_ZERO_TAPS");
+    if (off && off[0] == '0')
+        return;
+    if (fs == 7)
+        plan_up2x_taps_fs<7>(t, u);
+    else if (fs == 9)
+        plan_up2x_taps_fs<9>(t, u);
+}
+
 } // namespace
 
 int jinc_table_build_device(jinc_table* t, const double* lut)
@@ -765,6 +823,7 @@ int jinc_table_build_device(jinc_table* t, const double* lut)
                                   cudaMemcpyDeviceToHost, st));
     }
     JINC_CUDA(cudaStreamSynchronize(st));
+    plan_up2x_taps(t);
     if (n_blocks > 0 && (s.fs & 3) != 0) {
         // the strip role and the general kernel read weight rows as 16-byte vectors: a second copy with padded rows,
         // [block][fs][fsp], while it fits the budget (many-phase tables reach 65536 blocks)
@@ -884,6 +943,7 @@ extern "C" int jinc_table_get_info(const jinc_table* t, jinc_table_info* info)
     info->interior_y1 = t->iy1;
     info->filter_support = t->sc.support;
     info->build_ms = t->build_ms;
+    info->up2x_taps = t->fast_path == JINC_PATH_UP2X ? t->up2x.live_taps : 0;
     return JINC_OK;
 }
 

@@ -4,8 +4,10 @@
 #define JINC_UP2X_CUH
 
 #include <cstdlib>
+#include <utility>
 
 #include "jinc_resample.cuh"
+#include "jinc_up2x_taps.h"
 
 namespace jinc_rs {
 
@@ -50,8 +52,9 @@ __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity)
 }
 
 // One pair row of the tile applied to the thread's 16 accumulators: phase row 0 uses weight row rr, phase row 1 uses
-// weight row rr - OY1.
-template <int FS, int OX1, int OY1>
+// weight row rr - OY1.  Bit lx of C<py><px> clear: column lx of that phase's weight row is exactly zero and emits no FFMA2
+// (nor the LDS of a pair column no live tap reads); the remaining taps keep their order.
+template <int FS, int OX1, int OY1, uint32_t C00 = ~0u, uint32_t C01 = ~0u, uint32_t C10 = ~0u, uint32_t C11 = ~0u>
 __device__ __forceinline__ void up_row(const float2* __restrict__ trow, int rr, const UpWeights<FS>& W, float2 (&acc)[2][2][UP_TX])
 {
     using G = UpGeom<FS>;
@@ -66,8 +69,10 @@ __device__ __forceinline__ void up_row(const float2* __restrict__ trow, int rr, 
             const float w0 = W.w[0][0][rr][lx], w1 = W.w[0][1][rr][lx];
 #pragma unroll
             for (int i = 0; i < UP_TX; ++i) {
-                acc[0][0][i] = __ffma2_rn(seg[i + lx], make_float2(w0, w0), acc[0][0][i]);
-                acc[0][1][i] = __ffma2_rn(seg[i + OX1 + lx], make_float2(w1, w1), acc[0][1][i]);
+                if ((C00 >> lx) & 1)
+                    acc[0][0][i] = __ffma2_rn(seg[i + lx], make_float2(w0, w0), acc[0][0][i]);
+                if ((C01 >> lx) & 1)
+                    acc[0][1][i] = __ffma2_rn(seg[i + OX1 + lx], make_float2(w1, w1), acc[0][1][i]);
             }
         }
     }
@@ -78,14 +83,28 @@ __device__ __forceinline__ void up_row(const float2* __restrict__ trow, int rr, 
             const float w0 = W.w[1][0][ly1][lx], w1 = W.w[1][1][ly1][lx];
 #pragma unroll
             for (int i = 0; i < UP_TX; ++i) {
-                acc[1][0][i] = __ffma2_rn(seg[i + lx], make_float2(w0, w0), acc[1][0][i]);
-                acc[1][1][i] = __ffma2_rn(seg[i + OX1 + lx], make_float2(w1, w1), acc[1][1][i]);
+                if ((C10 >> lx) & 1)
+                    acc[1][0][i] = __ffma2_rn(seg[i + lx], make_float2(w0, w0), acc[1][0][i]);
+                if ((C11 >> lx) & 1)
+                    acc[1][1][i] = __ffma2_rn(seg[i + OX1 + lx], make_float2(w1, w1), acc[1][1][i]);
             }
         }
     }
 }
 
-template <typename T, int FS, int OX1, int OY1, bool TMA = false>
+// Every pair row of a small window, each with the live columns of tap-mask variant M as compile-time constants (a mask
+// read inside a run-time row loop would keep that loop rolled)
+template <int FS, int OX1, int OY1, int M, int... RR>
+__device__ __forceinline__ void up_rows(const float2* __restrict__ trow, const UpWeights<FS>& W, float2 (&acc)[2][2][UP_TX],
+                                        std::integer_sequence<int, RR...>)
+{
+    using K = UpTaps<FS, M>;
+    (up_row<FS, OX1, OY1, K::cols(0, 0, RR), K::cols(0, 1, RR), K::cols(1, 0, RR - OY1), K::cols(1, 1, RR - OY1)>(
+         trow + RR * UpGeom<FS>::NCP, RR, W, acc),
+     ...);
+}
+
+template <typename T, int FS, int OX1, int OY1, bool TMA = false, int M = 0>
 __global__ void __launch_bounds__(UP_THREADS, (FS >= 13 ? 4 : FS <= 7 ? 5 : 6))
     resample_up2x(const __grid_constant__ UpArgs a, const __grid_constant__ UpWeights<FS> W)
 {
@@ -238,10 +257,9 @@ __global__ void __launch_bounds__(UP_THREADS, (FS >= 13 ? 4 : FS <= 7 ? 5 : 6))
         if constexpr (FS <= UP_UNROLL_MAX_FS) {
             // small windows: the row loop is unrolled completely, so every weight has a fixed constant-bank address
             // and there is no loop control between the FFMA2 runs
-#pragma unroll
-            for (int rr = 0; rr < FS + OY1; ++rr)
-                up_row<FS, OX1, OY1>(trow + rr * G::NCP, rr, W, acc);
+            up_rows<FS, OX1, OY1, M>(trow, W, acc, std::make_integer_sequence<int, FS + OY1>{});
         } else {
+            static_assert(M == 0, "tap masks need the unrolled row loop");
 #pragma unroll 1
             for (int rr = 0; rr < FS + OY1; ++rr, trow += G::NCP)
                 up_row<FS, OX1, OY1>(trow, rr, W, acc);
@@ -282,7 +300,8 @@ __global__ void __launch_bounds__(UP_THREADS, (FS >= 13 ? 4 : FS <= 7 ? 5 : 6))
 // float planes staged by the bulk-copy engine: instantiated in its own translation unit (jinc_up2x_f32_bulk.cu)
 int launch_up2x_bulkcopy(const jinc_table* t, UpArgs& a, long long strip_blocks, int n_frames, cudaStream_t st);
 
-template <typename T, int FS, bool TMA>
+// M = 0: every tap, for the table's (ox1, oy1); M > 0: the tap-mask variant UpTaps<FS, M>, whose (ox1, oy1) the table has
+template <typename T, int FS, bool TMA, int M = 0>
 int launch_up2x_fs(const jinc_table* t, UpArgs& a, long long strip_blocks, int n_frames, cudaStream_t st)
 {
     using G = UpGeom<FS>;
@@ -296,8 +315,12 @@ int launch_up2x_fs(const jinc_table* t, UpArgs& a, long long strip_blocks, int n
                 for (int lx = 0; lx < FS; ++lx)
                     w.w[py][px][ly][lx] = blk[ly * FS + lx];
         }
-    auto kern = u.ox1 ? (u.oy1 ? resample_up2x<T, FS, 1, 1, TMA> : resample_up2x<T, FS, 1, 0, TMA>)
-                      : (u.oy1 ? resample_up2x<T, FS, 0, 1, TMA> : resample_up2x<T, FS, 0, 0, TMA>);
+    void (*kern)(UpArgs, UpWeights<FS>);
+    if constexpr (M == 0)
+        kern = u.ox1 ? (u.oy1 ? resample_up2x<T, FS, 1, 1, TMA> : resample_up2x<T, FS, 1, 0, TMA>)
+                     : (u.oy1 ? resample_up2x<T, FS, 0, 1, TMA> : resample_up2x<T, FS, 0, 0, TMA>);
+    else
+        kern = resample_up2x<T, FS, UpTaps<FS, M>::OX1, UpTaps<FS, M>::OY1, TMA, M>;
     size_t smem = G::SMEM;
     if constexpr (TMA)
         smem = UpTma<FS>::SMEM;
@@ -328,9 +351,40 @@ int launch_up2x_any(const jinc_table* t, UpArgs& a, long long strip_blocks, int 
     }
 }
 
+// integer planes of a table with a tap-mask variant (Up2xPlan::taps): one translation unit per (type, fs),
+// jinc_up2x_taps_<type>_fs<fs>.cu
+template <typename T, int FS>
+int launch_up2x_taps(const jinc_table* t, UpArgs& a, long long strip_blocks, int n_frames, cudaStream_t st)
+{
+    switch (t->up2x.taps) {
+    case 1: return launch_up2x_fs<T, FS, false, 1>(t, a, strip_blocks, n_frames, st);
+    case 2: return launch_up2x_fs<T, FS, false, 2>(t, a, strip_blocks, n_frames, st);
+    case 3: return launch_up2x_fs<T, FS, false, 3>(t, a, strip_blocks, n_frames, st);
+    case 4: return launch_up2x_fs<T, FS, false, 4>(t, a, strip_blocks, n_frames, st);
+    case 5: return launch_up2x_fs<T, FS, false, 5>(t, a, strip_blocks, n_frames, st);
+    case 6: return launch_up2x_fs<T, FS, false, 6>(t, a, strip_blocks, n_frames, st);
+    case 7: return launch_up2x_fs<T, FS, false, 7>(t, a, strip_blocks, n_frames, st);
+    default: return jinc_fail(JINC_E_INVALID, "resample_up2x: no tap-mask variant %d for fs %d", t->up2x.taps, FS);
+    }
+}
+static_assert(UP_TAP_VARIANTS == 8, "launch_up2x_taps dispatches variants 1..7");
+extern template int launch_up2x_taps<uint8_t, 7>(const jinc_table*, UpArgs&, long long, int, cudaStream_t);
+extern template int launch_up2x_taps<uint8_t, 9>(const jinc_table*, UpArgs&, long long, int, cudaStream_t);
+extern template int launch_up2x_taps<uint16_t, 7>(const jinc_table*, UpArgs&, long long, int, cudaStream_t);
+extern template int launch_up2x_taps<uint16_t, 9>(const jinc_table*, UpArgs&, long long, int, cudaStream_t);
+
 template <typename T>
 int launch_up2x(const jinc_table* t, UpArgs& a, long long strip_blocks, int n_frames, cudaStream_t st)
 {
+    if constexpr (sizeof(T) < 4) {
+        // float planes always take every tap: 0 * Inf and 0 * NaN must reach the output as they do in the reference
+        if (t->up2x.taps > 0) {
+            if (t->sc.fs == 7)
+                return launch_up2x_taps<T, 7>(t, a, strip_blocks, n_frames, st);
+            if (t->sc.fs == 9)
+                return launch_up2x_taps<T, 9>(t, a, strip_blocks, n_frames, st);
+        }
+    }
     if constexpr (sizeof(T) == 4) {
         const char* tma_env = getenv("JINCRESIZE_B200_TMA");
         if (tma_env && tma_env[0] == '1' && up2x_supported(t->sc.fs)) {

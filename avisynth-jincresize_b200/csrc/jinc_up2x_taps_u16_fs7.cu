@@ -1,0 +1,6 @@
+// exact-2x interior kernels of uint16_t planes, fs 7, with the zero taps of a tap-mask variant skipped
+#include "jinc_up2x.cuh"
+
+namespace jinc_rs {
+template int launch_up2x_taps<uint16_t, 7>(const jinc_table*, UpArgs&, long long, int, cudaStream_t);
+}

@@ -32,7 +32,8 @@ class TableInfo(C.Structure):
     _fields_ = [("filter_size", C.c_int32), ("n_phase_x", C.c_int32), ("n_phase_y", C.c_int32),
                 ("n_border_cols", C.c_int32), ("n_border_rows", C.c_int32), ("fast_path", C.c_int32),
                 ("interior_x0", C.c_int32), ("interior_x1", C.c_int32), ("interior_y0", C.c_int32),
-                ("interior_y1", C.c_int32), ("filter_support", C.c_float), ("build_ms", C.c_float)]
+                ("interior_y1", C.c_int32), ("filter_support", C.c_float), ("build_ms", C.c_float),
+                ("up2x_taps", C.c_int32)]
 
 
 class FilterParams(C.Structure):

@@ -96,6 +96,8 @@ typedef struct jinc_table_info {
     float filter_support;  /* src/JincResize.cpp:355 */
     float build_ms;        /* host wall time of jinc_table_create: LUT + device kernels + plans (the reference's
                               generate_coeff_table_c call, src/JincResize.cpp:829,864) */
+    int32_t up2x_taps;     /* JINC_PATH_UP2X: taps per 2x2 output cell the kernel multiplies on 8/16-bit planes (4 * fs^2
+                              unless exactly-zero taps are skipped); 0 on the other paths */
 } jinc_table_info;
 
 JINC_API int jinc_table_create(jinc_ctx* ctx, const jinc_table_params* p, jinc_table** out);
