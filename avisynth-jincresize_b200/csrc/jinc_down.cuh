@@ -29,6 +29,10 @@ __device__ __forceinline__ void down_pack(float2& out, const float* r0, const fl
 {
     out = make_float2(__ldg(r0), __ldg(r1));
 }
+__device__ __forceinline__ void down_pack(float2& out, const __half* r0, const __half* r1, int)
+{
+    out = make_float2(__half2float(__ldg(r0)), __half2float(__ldg(r1)));
+}
 
 template <typename T, int N>
 __device__ __forceinline__ void store_run(T* p, const float (&v)[N], float peak)
@@ -36,9 +40,11 @@ __device__ __forceinline__ void store_run(T* p, const float (&v)[N], float peak)
     static_assert(N % 4 == 0, "runs are multiples of four samples");
 #pragma unroll
     for (int q = 0; q < N; q += 4) {
-        if (sizeof(T) == 4) {
+        if constexpr (std::is_same<T, float>::value) {
             *reinterpret_cast<float4*>(p + q) = make_float4(v[q], v[q + 1], v[q + 2], v[q + 3]);
-        } else if (sizeof(T) == 2) {
+        } else if constexpr (std::is_same<T, __half>::value) {
+            *reinterpret_cast<uint2*>(p + q) = make_uint2(pack_half2(v[q], v[q + 1]), pack_half2(v[q + 2], v[q + 3]));
+        } else if constexpr (sizeof(T) == 2) {
             *reinterpret_cast<uint2*>(p + q) = make_uint2(finish_u16(v[q], peak) | (finish_u16(v[q + 1], peak) << 16),
                                                           finish_u16(v[q + 2], peak) | (finish_u16(v[q + 3], peak) << 16));
         } else {
@@ -257,7 +263,7 @@ int launch_down_fs(const jinc_table* t, DownArgs& a, const int* wblocks, bool wa
     static_assert(NPASS <= DN_MAX_PASSES, "too many passes");
     DownWeightsN<FS, Q, NPASS> w;
     memset(&w, 0, sizeof(w));
-    const int bits = sizeof(T) == 4 ? 32 : t_bits_from_peak(a.fr.peak);
+    const int bits = is_float_sample<T>::value ? 32 : t_bits_from_peak(a.fr.peak);
     for (int ps = 0; ps < NPASS; ++ps) {
         const float* blk = t->h_weights.data() + (size_t)wblocks[ps] * FS * FS;
         // set 0 pairs rows (2k, 2k+1); set 1 (odd ratios) pairs rows (2k-1, 2k); sums per half for the PRMT bias
@@ -285,7 +291,7 @@ int launch_down_fs(const jinc_table* t, DownArgs& a, const int* wblocks, bool wa
             a.pass[ps].bias_y[j] = (float)(0.5 * sum_y[j]);
         }
     }
-    if constexpr (sizeof(T) == 4) {
+    if constexpr (is_float_sample<T>::value) { // half planes are staged as float pairs too
         return launch_down_cfg<T, FS, Q, DN_NX, DN_NY, DN_CVT_FLOAT, NPASS>(t, a, w, want_strips, n_frames, st, rects, n_rects);
     } else {
         if (bits <= 15) {

@@ -297,7 +297,7 @@ int enqueue_frame(jinc_filter* f, Slot* s, const jinc_frame* frame, int y0_luma,
 {
     DeviceState& d = f->devs[s->dev_index];
     JINC_CUDA(cudaSetDevice(d.ctx->device));
-    const int sb = f->p.sample_bytes;
+    const int sb = jinc_sample_size(f->p.sample_bytes); // bytes per sample
     const int np = f->p.n_planes;
     const bool may_register = (f->p.flags & JINC_FILTER_HOST_REGISTER) != 0;
     s->probe_active = false;
@@ -476,7 +476,8 @@ int enqueue_frame(jinc_filter* f, Slot* s, const jinc_frame* frame, int y0_luma,
         if (n == 0)
             continue;
         int launched = 0;
-        const int rc = jinc_launch_resize_planes(d.ctx, d.tables[k], sb, f->peak, n, src, sp, dst, dp, yb, ye, s->stream, &launched);
+        const int rc = jinc_launch_resize_planes(d.ctx, d.tables[k], f->p.sample_bytes, f->peak, n, src, sp, dst, dp, yb, ye, s->stream,
+                                                  &launched);
         f->launches.fetch_add(launched);
         if (rc != JINC_OK)
             return rc;
@@ -549,7 +550,7 @@ int finish_frame(jinc_filter* f, Slot* s, int y0_luma, int y1_luma, bool whole)
     DeviceState& d = f->devs[s->dev_index];
     JINC_CUDA(cudaSetDevice(d.ctx->device));
     JINC_CUDA(cudaEventSynchronize(s->done));
-    const int sb = f->p.sample_bytes;
+    const int sb = jinc_sample_size(f->p.sample_bytes); // bytes per sample
     if (s->probe_active) {
         // what the GPU received through the registration against what the caller's memory holds now
         const uint32_t n_words = static_cast<uint32_t>(f->src_bytes / 4);
@@ -709,11 +710,13 @@ extern "C" int jinc_filter_create(const jinc_filter_params* p, jinc_filter** out
     *out = nullptr;
     if (p->n_planes < 1 || p->n_planes > JINC_MAX_PLANES)
         return jinc_fail(JINC_E_INVALID, "jinc_filter_create: n_planes must be 1..4");
-    if (p->sample_bytes != 1 && p->sample_bytes != 2 && p->sample_bytes != 4)
-        return jinc_fail(JINC_E_INVALID, "jinc_filter_create: sample_bytes must be 1, 2 or 4");
+    if (!jinc_sample_valid(p->sample_bytes))
+        return jinc_fail(JINC_E_INVALID, "jinc_filter_create: sample_bytes must be 1, 2, 4 or JINC_SAMPLE_F16");
     // bits feed peak = (1 << bits) - 1 (:793): 8 for one-byte samples, 10..16 for two-byte samples; float ignores it
     if ((p->sample_bytes == 1 && p->bits != 8) || (p->sample_bytes == 2 && (p->bits < 9 || p->bits > 16)))
         return jinc_fail(JINC_E_INVALID, "jinc_filter_create: %d bits per component do not fit %d-byte samples", p->bits, p->sample_bytes);
+    if (p->sample_bytes == JINC_SAMPLE_F16 && p->bits != 16)
+        return jinc_fail(JINC_E_INVALID, "jinc_filter_create: %d bits per component do not fit half (16-bit float) samples", p->bits);
     if (p->tap < 1 || p->tap > 16)
         return jinc_fail(JINC_E_INVALID, "JincResize: tap must be between 1..16.");
     if (p->src_w < 1 || p->src_h < 1 || p->target_w < 1 || p->target_h < 1)
@@ -744,7 +747,7 @@ extern "C" int jinc_filter_create(const jinc_filter_params* p, jinc_filter** out
         jinc_hostmem::client_add();
         f->registers = true;
     }
-    f->peak = (p->sample_bytes == 4) ? 0.f : static_cast<float>((1 << p->bits) - 1); // :793
+    f->peak = jinc_sample_is_float(p->sample_bytes) ? 0.f : static_cast<float>((1 << p->bits) - 1); // :793
     derive_table_params(*p, f->tparams, &f->n_tables);
 
     // Plane layout shared by device and pinned buffers: 64-byte pitches and 64-byte plane offsets.  Vector loads/stores
@@ -759,8 +762,8 @@ extern "C" int jinc_filter_create(const jinc_filter_params* p, jinc_filter** out
         pl.src_h = tp.src_h;
         pl.dst_w = tp.dst_w;
         pl.dst_h = tp.dst_h;
-        pl.src_pitch = align_up(static_cast<size_t>(pl.src_w) * p->sample_bytes, 64);
-        pl.dst_pitch = align_up(static_cast<size_t>(pl.dst_w) * p->sample_bytes, 64);
+        pl.src_pitch = align_up(static_cast<size_t>(pl.src_w) * jinc_sample_size(p->sample_bytes), 64);
+        pl.dst_pitch = align_up(static_cast<size_t>(pl.dst_w) * jinc_sample_size(p->sample_bytes), 64);
         pl.src_off = so;
         pl.dst_off = dof;
         so += pl.src_pitch * pl.src_h;

@@ -204,22 +204,28 @@ int jinc_table_build_device(jinc_table* t, const double* lut);
 cudaError_t jinc_gather_blocks(float* out, const uint32_t* list, unsigned n, const float* phase_blocks, const float* border_blocks,
                                int block_floats, cudaStream_t st);
 
+// Sample format of the C ABI (the `sample_bytes` arguments): 1 (uint8), 2 (uint16), 4 (float) or JINC_SAMPLE_F16 (IEEE
+// binary16).  The launchers below take this code; byte counts (pitches, plane sizes, transfers) take jinc_sample_size.
+inline bool jinc_sample_valid(int sample) { return sample == 1 || sample == 2 || sample == 4 || sample == JINC_SAMPLE_F16; }
+inline int jinc_sample_size(int sample) { return sample & 0xff; }
+inline bool jinc_sample_is_float(int sample) { return sample == 4 || sample == JINC_SAMPLE_F16; }
+
 // jinc_resize.cu
 int jinc_build_strip_plan(jinc_table* t); // after plan_fast_paths and the weight blocks; no plan is not an error
 void jinc_free_strip_plan(jinc_table* t);
-int jinc_launch_resize(jinc_ctx* ctx, const jinc_table* t, int sample_bytes, float peak, const void* d_src,
+int jinc_launch_resize(jinc_ctx* ctx, const jinc_table* t, int sample, float peak, const void* d_src,
                        ptrdiff_t src_pitch, void* d_dst, ptrdiff_t dst_pitch, int y_begin, int y_end,
                        cudaStream_t stream, int* launches);
 // several planes that share one table in a single launch (blockIdx.z / .y = plane); rows [y_begin,y_end)
-int jinc_launch_resize_planes(jinc_ctx* ctx, const jinc_table* t, int sample_bytes, float peak, int n_planes,
+int jinc_launch_resize_planes(jinc_ctx* ctx, const jinc_table* t, int sample, float peak, int n_planes,
                               const void* const* d_src, const ptrdiff_t* src_pitch, void* const* d_dst,
                               const ptrdiff_t* dst_pitch, int y_begin, int y_end, cudaStream_t stream, int* launches,
                               int parts = JINC_PART_ALL);
 // batched: d_frame_ptrs is a DEVICE array of n_frames packed plane-pointer records (jinc_pack_plane_ptrs)
 size_t jinc_plane_ptrs_size();
-int jinc_pack_plane_ptrs(void* out, int sample_bytes, int n_planes, const void* const* d_src, const ptrdiff_t* src_pitch,
+int jinc_pack_plane_ptrs(void* out, int sample, int n_planes, const void* const* d_src, const ptrdiff_t* src_pitch,
                          void* const* d_dst, const ptrdiff_t* dst_pitch);
-int jinc_launch_resize_batch(jinc_ctx* ctx, const jinc_table* t, int sample_bytes, float peak, int n_planes,
+int jinc_launch_resize_batch(jinc_ctx* ctx, const jinc_table* t, int sample, float peak, int n_planes,
                              const void* d_frame_ptrs, int n_frames, cudaStream_t stream, int* launches, int parts);
 int jinc_debug_pixel_weights(const jinc_table* t, int x, int y, float* out);
 // probe words of a device buffer: d_out[k] = 32-bit word jinc_probe_index(seed, k, n_words) of d_buf, k < JINC_PROBE_WORDS

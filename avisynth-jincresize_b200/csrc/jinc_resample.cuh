@@ -40,12 +40,22 @@
 #include <type_traits>
 #include <vector>
 
+#include <cuda_fp16.h>
+
 #include "jinc_internal.h"
 #include "jinc_weights.cuh"
 
 namespace jinc_rs {
 
 // ------------------------------------------------------------------------------------------ sample conversion
+//
+// Four sample types: uint8_t, uint16_t (9..16 bits), float and __half (IEEE binary16).  Float planes -- float and half --
+// keep the raw sum (no clamp, NaN and Inf propagated) and multiply every tap; half is converted to float when it is
+// staged and rounded to nearest-even when it is stored, so a half plane runs the float inner loops unchanged.  Kernels
+// tell the two kinds apart with is_float_sample, never with sizeof: a half is as wide as a uint16_t.
+template <typename T>
+struct is_float_sample : std::integral_constant<bool, std::is_same<T, float>::value || std::is_same<T, __half>::value> {
+};
 
 // clamp to [0, peak] and round half to even (lrintf) in one saturating convert; NaN -> 0
 // (8-bit planes always have peak = 255, which the saturating convert already enforces)
@@ -86,6 +96,22 @@ __device__ __forceinline__ uint16_t finish<uint16_t>(float v, float peak)
 {
     return (uint16_t)finish_u16(v, peak);
 }
+// round to nearest even, no clamp: sums of magnitude >= 65520 become +-Inf
+template <>
+__device__ __forceinline__ __half finish<__half>(float v, float)
+{
+    return __float2half_rn(v);
+}
+// two halves in one word, the first in the low 16 bits (the lower address)
+__device__ __forceinline__ uint32_t pack_half2(float lo, float hi)
+{
+    return (uint32_t)__half_as_ushort(__float2half_rn(lo)) | ((uint32_t)__half_as_ushort(__float2half_rn(hi)) << 16);
+}
+// one half of a word as float (exact, subnormals included)
+__device__ __forceinline__ float half_bits_to_float(uint32_t w, int hi)
+{
+    return __half2float(__ushort_as_half((unsigned short)(hi ? w >> 16 : w & 0xffffu)));
+}
 
 // Integer samples become floats without the (quarter-rate) I2F: drop the bits into the mantissa of 2^23 and subtract
 // 2^23 again -- exact for any value below 2^23.
@@ -99,6 +125,11 @@ __device__ __forceinline__ float load_sample<float>(const float* p)
 {
     return __ldg(p);
 }
+template <>
+__device__ __forceinline__ float load_sample<__half>(const __half* p)
+{
+    return __half2float(__ldg(p));
+}
 template <typename T>
 __device__ __forceinline__ float sample_to_float(T v)
 {
@@ -108,6 +139,11 @@ template <>
 __device__ __forceinline__ float sample_to_float<float>(float v)
 {
     return v;
+}
+template <>
+__device__ __forceinline__ float sample_to_float<__half>(__half v)
+{
+    return __half2float(v);
 }
 
 // four consecutive samples as one aligned vector load
@@ -124,6 +160,10 @@ struct Vec4Of<uint16_t> {
 template <>
 struct Vec4Of<float> {
     using type = float4;
+};
+template <>
+struct Vec4Of<__half> {
+    using type = uint2;
 };
 // sample k (0..3, a constant after unrolling) of such a group as float: integer samples are dropped into the mantissa
 // of 2^23 by one byte permute, then 2^23 is subtracted
@@ -144,6 +184,11 @@ __device__ __forceinline__ float vec4_sample<float>(const float4& v, int k)
 {
     return k == 0 ? v.x : k == 1 ? v.y : k == 2 ? v.z : v.w;
 }
+template <>
+__device__ __forceinline__ float vec4_sample<__half>(const uint2& v, int k)
+{
+    return half_bits_to_float((k & 2) ? v.y : v.x, k & 1);
+}
 
 template <typename T>
 __device__ __forceinline__ void store8(T* p, const float (&v)[8], float peak);
@@ -152,6 +197,11 @@ __device__ __forceinline__ void store8<float>(float* p, const float (&v)[8], flo
 {
     reinterpret_cast<float4*>(p)[0] = make_float4(v[0], v[1], v[2], v[3]);
     reinterpret_cast<float4*>(p)[1] = make_float4(v[4], v[5], v[6], v[7]);
+}
+template <>
+__device__ __forceinline__ void store8<__half>(__half* p, const float (&v)[8], float)
+{
+    *reinterpret_cast<uint4*>(p) = make_uint4(pack_half2(v[0], v[1]), pack_half2(v[2], v[3]), pack_half2(v[4], v[5]), pack_half2(v[6], v[7]));
 }
 template <>
 __device__ __forceinline__ void store8<uint16_t>(uint16_t* p, const float (&v)[8], float peak)
@@ -257,7 +307,8 @@ __device__ __forceinline__ const PlanePtrs& frame_ptrs(const FrameSet& fs)
 }
 
 // Window rows as aligned 32-bit words (the plane base and pitch are 4-byte aligned), converted later: the words are
-// funnel-shifted into place and every sample is dropped into the mantissa of 2^23 by one byte permute.
+// funnel-shifted into place and every integer sample is dropped into the mantissa of 2^23 by one byte permute (a half
+// sample is converted as it is).
 template <typename T, int FS>
 struct RowWords {
     static constexpr int SB = (int)sizeof(T);
@@ -300,12 +351,16 @@ __device__ __forceinline__ void row_words_to_float(const uint32_t (&w)[RowWords<
             al[j] = __funnelshift_r(w[j], w[j + 1], off * 8);
 #pragma unroll
         for (int i = 0; i < FS; ++i) {
-            uint32_t bits;
-            if (R::SB == 1)
-                bits = __byte_perm(al[i >> 2], 0x4B000000u, 0x7440 | (i & 3));
-            else
-                bits = __byte_perm(al[i >> 1], 0x4B000000u, (i & 1) ? 0x7432 : 0x7410);
-            v[i] = __uint_as_float(bits) - 8388608.f;
+            if constexpr (is_float_sample<T>::value) {
+                v[i] = half_bits_to_float(al[i >> 1], i & 1);
+            } else {
+                uint32_t bits;
+                if (R::SB == 1)
+                    bits = __byte_perm(al[i >> 2], 0x4B000000u, 0x7440 | (i & 3));
+                else
+                    bits = __byte_perm(al[i >> 1], 0x4B000000u, (i & 1) ? 0x7432 : 0x7410);
+                v[i] = __uint_as_float(bits) - 8388608.f;
+            }
         }
     }
 }
@@ -1431,7 +1486,7 @@ enum { DN_CVT_I2F = 0, DN_CVT_PRMT = 1, DN_CVT_FLOAT = 2 };
 
 template <typename T, int FS, int Q, int NX, int NY>
 struct DownGeom {
-    static constexpr bool IS_FLOAT = sizeof(T) == 4;
+    static constexpr bool IS_FLOAT = is_float_sample<T>::value; // float and half planes: float pairs, half-height tiles
     using Word = typename std::conditional<IS_FLOAT, float2, uint32_t>::type; // {row 2k, row 2k+1}
     static constexpr int LX = DN_TW / NX;               // lanes along x
     static constexpr int LY = 32 / LX;                  // lanes along y

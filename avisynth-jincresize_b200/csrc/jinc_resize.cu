@@ -490,10 +490,13 @@ int launch_typed(const jinc_table* t, const FrameSet& fr, int n_frames, int y_be
     return JINC_OK;
 }
 
-int check_and_fill(PlanePtrs& pl, int sample_bytes, int n_planes, const void* const* d_src, const ptrdiff_t* src_pitch,
+int check_and_fill(PlanePtrs& pl, int sample, int n_planes, const void* const* d_src, const ptrdiff_t* src_pitch,
                    void* const* d_dst, const ptrdiff_t* dst_pitch)
 {
     memset(&pl, 0, sizeof(pl));
+    if (!jinc_sample_valid(sample))
+        return jinc_fail(JINC_E_INVALID, "resize: sample_bytes must be 1, 2, 4 or JINC_SAMPLE_F16");
+    const int sample_bytes = jinc_sample_size(sample);
     for (int i = 0; i < n_planes; ++i) {
         if (!d_src[i] || !d_dst[i])
             return jinc_fail(JINC_E_INVALID, "resize: null plane pointer");
@@ -509,7 +512,7 @@ int check_and_fill(PlanePtrs& pl, int sample_bytes, int n_planes, const void* co
     return JINC_OK;
 }
 
-int dispatch(const jinc_table* t, int sample_bytes, const FrameSet& fr, int n_frames, int y_begin, int y_end, cudaStream_t stream,
+int dispatch(const jinc_table* t, int sample, const FrameSet& fr, int n_frames, int y_begin, int y_end, cudaStream_t stream,
              int* launches, int parts)
 {
     y_begin = std::max(y_begin, 0);
@@ -519,11 +522,12 @@ int dispatch(const jinc_table* t, int sample_bytes, const FrameSet& fr, int n_fr
     int dummy = 0;
     if (!launches)
         launches = &dummy;
-    switch (sample_bytes) {
+    switch (sample) {
     case 1: return launch_typed<uint8_t>(t, fr, n_frames, y_begin, y_end, stream, launches, parts);
     case 2: return launch_typed<uint16_t>(t, fr, n_frames, y_begin, y_end, stream, launches, parts);
     case 4: return launch_typed<float>(t, fr, n_frames, y_begin, y_end, stream, launches, parts);
-    default: return jinc_fail(JINC_E_INVALID, "resize: sample_bytes must be 1, 2 or 4");
+    case JINC_SAMPLE_F16: return launch_typed<__half>(t, fr, n_frames, y_begin, y_end, stream, launches, parts);
+    default: return jinc_fail(JINC_E_INVALID, "resize: sample_bytes must be 1, 2, 4 or JINC_SAMPLE_F16");
     }
 }
 
@@ -873,8 +877,8 @@ int jinc_build_strip_plan(jinc_table* t)
         const size_t smem = (size_t)fhc * (size_t)(d * ((fwc + d - 1) / d)) * sizeof(float); // CellsGeom<FS, Q>::SMEM
         pp = StripPlanParams{32 * warps, CL_STRIP_SPT, t->cells.ax[0].P, t->cells.ax[1].P, q, (unsigned)(smem / sizeof(float))};
     } else if (t->fast_path == JINC_PATH_DOWN_INT && down_supported(t)) {
-        // DownGeom<T, FS, Q, 8, 2> of the integer sample types (128 threads per block; float planes run 64-thread blocks and
-        // keep the prologue path): a lower bound of its shared memory (the row padding left out)
+        // DownGeom<T, FS, Q, 8, 2> of the integer sample types (128 threads per block; float and half planes run 64-thread
+        // blocks and keep the prologue path): a lower bound of its shared memory (the row padding left out)
         const int q = t->down.qx;
         const int nkw1 = (q & 1) ? (fs + 2) / 2 : ((fs + 1) & ~1) / 2;
         const int nrowp = (q * (DN_TH - 1) + 2 * nkw1 + 1) / 2, mt = (fs + q - 1) / q, d = q * 8;
@@ -931,15 +935,15 @@ int jinc_build_strip_plan(jinc_table* t)
     return JINC_OK;
 }
 
-int jinc_pack_plane_ptrs(void* out, int sample_bytes, int n_planes, const void* const* d_src, const ptrdiff_t* src_pitch,
+int jinc_pack_plane_ptrs(void* out, int sample, int n_planes, const void* const* d_src, const ptrdiff_t* src_pitch,
                          void* const* d_dst, const ptrdiff_t* dst_pitch)
 {
     if (n_planes < 1 || n_planes > JINC_MAX_PLANES)
         return jinc_fail(JINC_E_INVALID, "resize: n_planes must be 1..4");
-    return check_and_fill(*static_cast<PlanePtrs*>(out), sample_bytes, n_planes, d_src, src_pitch, d_dst, dst_pitch);
+    return check_and_fill(*static_cast<PlanePtrs*>(out), sample, n_planes, d_src, src_pitch, d_dst, dst_pitch);
 }
 
-int jinc_launch_resize_planes(jinc_ctx* ctx, const jinc_table* t, int sample_bytes, float peak, int n_planes,
+int jinc_launch_resize_planes(jinc_ctx* ctx, const jinc_table* t, int sample, float peak, int n_planes,
                               const void* const* d_src, const ptrdiff_t* src_pitch, void* const* d_dst,
                               const ptrdiff_t* dst_pitch, int y_begin, int y_end, cudaStream_t stream, int* launches,
                               int parts)
@@ -947,15 +951,15 @@ int jinc_launch_resize_planes(jinc_ctx* ctx, const jinc_table* t, int sample_byt
     (void)ctx;
     FrameSet fr;
     memset(&fr, 0, sizeof(fr));
-    if (int rc = jinc_pack_plane_ptrs(&fr.one, sample_bytes, n_planes, d_src, src_pitch, d_dst, dst_pitch))
+    if (int rc = jinc_pack_plane_ptrs(&fr.one, sample, n_planes, d_src, src_pitch, d_dst, dst_pitch))
         return rc;
     fr.frames = nullptr;
     fr.n_planes = n_planes;
     fr.peak = peak;
-    return dispatch(t, sample_bytes, fr, 1, y_begin, y_end, stream, launches, parts);
+    return dispatch(t, sample, fr, 1, y_begin, y_end, stream, launches, parts);
 }
 
-int jinc_launch_resize_batch(jinc_ctx* ctx, const jinc_table* t, int sample_bytes, float peak, int n_planes,
+int jinc_launch_resize_batch(jinc_ctx* ctx, const jinc_table* t, int sample, float peak, int n_planes,
                              const void* d_frame_ptrs, int n_frames, cudaStream_t stream, int* launches, int parts)
 {
     (void)ctx;
@@ -964,14 +968,14 @@ int jinc_launch_resize_batch(jinc_ctx* ctx, const jinc_table* t, int sample_byte
     fr.frames = static_cast<const PlanePtrs*>(d_frame_ptrs);
     fr.n_planes = n_planes;
     fr.peak = peak;
-    return dispatch(t, sample_bytes, fr, n_frames, 0, t->sc.dst_h, stream, launches, parts);
+    return dispatch(t, sample, fr, n_frames, 0, t->sc.dst_h, stream, launches, parts);
 }
 
-int jinc_launch_resize(jinc_ctx* ctx, const jinc_table* t, int sample_bytes, float peak, const void* d_src,
+int jinc_launch_resize(jinc_ctx* ctx, const jinc_table* t, int sample, float peak, const void* d_src,
                        ptrdiff_t src_pitch, void* d_dst, ptrdiff_t dst_pitch, int y_begin, int y_end, cudaStream_t stream,
                        int* launches)
 {
-    return jinc_launch_resize_planes(ctx, t, sample_bytes, peak, 1, &d_src, &src_pitch, &d_dst, &dst_pitch, y_begin, y_end,
+    return jinc_launch_resize_planes(ctx, t, sample, peak, 1, &d_src, &src_pitch, &d_dst, &dst_pitch, y_begin, y_end,
                                      stream, launches, JINC_PART_ALL);
 }
 

@@ -142,7 +142,7 @@ __global__ void __launch_bounds__(UP_THREADS, (FS >= 13 ? 4 : FS <= 7 ? 5 : 6))
     //      (4 samples per LDG); the tile columns then start d = tsx & 3 samples into the first group.
     const bool vec_ok = ((reinterpret_cast<uintptr_t>(src) | (uintptr_t)(sp * (long long)sizeof(T))) & (4 * sizeof(T) - 1)) == 0;
     if constexpr (TMA) {
-        static_assert(sizeof(T) == 4, "bulk-copy staging lands float rows");
+        static_assert(std::is_same<T, float>::value, "bulk-copy staging lands float rows");
         // One cp.async.bulk per raw tile row (a contiguous, 16-byte aligned segment of the plane row: vec_ok is required by the
         // launcher), issued by the lanes of warp 0, all completing on one mbarrier.  The segment is cut at the end of the
         // plane row; what lies beyond only feeds discarded cells.
@@ -376,8 +376,8 @@ extern template int launch_up2x_taps<uint16_t, 9>(const jinc_table*, UpArgs&, lo
 template <typename T>
 int launch_up2x(const jinc_table* t, UpArgs& a, long long strip_blocks, int n_frames, cudaStream_t st)
 {
-    if constexpr (sizeof(T) < 4) {
-        // float planes always take every tap: 0 * Inf and 0 * NaN must reach the output as they do in the reference
+    if constexpr (!is_float_sample<T>::value) {
+        // float and half planes always take every tap: 0 * Inf and 0 * NaN must reach the output as they do in the reference
         if (t->up2x.taps > 0) {
             if (t->sc.fs == 7)
                 return launch_up2x_taps<T, 7>(t, a, strip_blocks, n_frames, st);
@@ -385,7 +385,7 @@ int launch_up2x(const jinc_table* t, UpArgs& a, long long strip_blocks, int n_fr
                 return launch_up2x_taps<T, 9>(t, a, strip_blocks, n_frames, st);
         }
     }
-    if constexpr (sizeof(T) == 4) {
+    if constexpr (std::is_same<T, float>::value) { // half planes ignore the switch: the landed rows are float rows
         const char* tma_env = getenv("JINCRESIZE_B200_TMA");
         if (tma_env && tma_env[0] == '1' && up2x_supported(t->sc.fs)) {
             // bulk-copy staging needs 16-byte aligned plane rows in every frame; batched launches (device-side plane

@@ -15,6 +15,8 @@ from . import paths
 MAX_PLANES = 4
 MAX_DEVICES = 16
 CPLACE = {"mpeg2": 0, "mpeg1": 1, "topleft": 2}
+SAMPLE_F16 = 0x102  # JINC_SAMPLE_F16: IEEE binary16 planes (numpy float16), passed where the ABI takes sample_bytes
+DTYPES = {1: np.uint8, 2: np.uint16, 4: np.float32, SAMPLE_F16: np.float16}
 PATH_NAMES = {0: "general", 1: "up2x", 2: "down_int", 3: "periodic", 4: "piecewise"}
 
 
@@ -254,6 +256,7 @@ class Table(TableView):
 
     def resize_device(self, sample_bytes: int, peak: float, d_src: int, src_pitch: int, d_dst: int, dst_pitch: int,
                       stream: int = 0):
+        """One device-resident plane; sample_bytes is 1, 2, 4 or SAMPLE_F16 (peak is then ignored)."""
         _check(lib().jinc_resize_plane_device(self.ctx.handle, self.handle, sample_bytes, peak, d_src, src_pitch,
                                               d_dst, dst_pitch, stream or None))
 
@@ -294,7 +297,7 @@ class Filter:
         h = C.c_void_p()
         _check(lib().jinc_filter_create(C.byref(p), C.byref(h)))
         self.handle = h
-        self.dtype = {1: np.uint8, 2: np.uint16, 4: np.float32}[sample_bytes]
+        self.dtype = DTYPES[sample_bytes]
 
     def plane_shapes(self):
         p = self.params

@@ -90,8 +90,9 @@ void VS_CC create(const VSMap* in, VSMap* out, void*, VSCore* core, const VSAPI*
     if (vi->format.colorFamily == cfUndefined || vi->width <= 0 || vi->height <= 0)
         return fail("JincResize: only constant format input is supported.");
     const bool is_float = vi->format.sampleType == stFloat;
-    if ((is_float && vi->format.bitsPerSample != 32) || (!is_float && (vi->format.bitsPerSample < 8 || vi->format.bitsPerSample > 16)))
-        return fail("JincResize: only 8..16 bit integer and 32 bit float input is supported.");
+    const bool is_half = is_float && vi->format.bitsPerSample == 16; // GRAYH, YUV4xxPH, RGBH
+    if ((is_float && vi->format.bitsPerSample != 32 && !is_half) || (!is_float && (vi->format.bitsPerSample < 8 || vi->format.bitsPerSample > 16)))
+        return fail("JincResize: only 8..16 bit integer, 16 bit float and 32 bit float input is supported.");
 
     const int tap = static_cast<int>(opt_int("tap", 3));
     if (tap < 1 || tap > 16)
@@ -154,7 +155,7 @@ void VS_CC create(const VSMap* in, VSMap* out, void*, VSCore* core, const VSAPI*
     p.blur = opt_float("blur", 0.0); // 0 => 1.0 inside the library (:772-774)
     p.cplace = cplace == "mpeg2" ? JINC_CPLACE_MPEG2 : (cplace == "mpeg1" ? JINC_CPLACE_MPEG1 : JINC_CPLACE_TOPLEFT);
     p.n_planes = vi->format.numPlanes;
-    p.sample_bytes = vi->format.bytesPerSample;
+    p.sample_bytes = is_half ? JINC_SAMPLE_F16 : vi->format.bytesPerSample; // the output format is the input format
     p.bits = vi->format.bitsPerSample;
     p.sub_w = subsampled ? vi->format.subSamplingW : 0;
     p.sub_h = subsampled ? vi->format.subSamplingH : 0;

@@ -37,6 +37,14 @@ enum {
     JINC_E_BUSY = -5     /* jinc_filter_try_submit: every in-flight slot is taken */
 };
 
+/* Sample format of an IEEE binary16 (half-precision float) plane, accepted wherever the ABI takes `sample_bytes`
+ * (jinc_filter_params.sample_bytes with bits = 16, jinc_resize_plane_device with peak ignored).  The low byte is the
+ * sample size.  Half planes are resampled like float planes: every sample is widened to float exactly, the sum is
+ * accumulated in float in the same order as for a float plane, and the result is rounded to the nearest half (ties to
+ * even) with no clamp: sums of magnitude 65520 or more become +-Inf, NaN and Inf inputs propagate.  So a half frame
+ * equals the float frame of the widened input, rounded to half. */
+#define JINC_SAMPLE_F16 0x102
+
 /* chroma sample location (src/JincResize.cpp:715-745; README "cplace") */
 enum { JINC_CPLACE_MPEG2 = 0, JINC_CPLACE_MPEG1 = 1, JINC_CPLACE_TOPLEFT = 2 };
 
@@ -123,8 +131,8 @@ JINC_API int jinc_table_pixel_block(const jinc_table* t, int x, int y, int64_t* 
 /* ---------------------------------------------------------------- resampling, device-resident planes
  * Replaces: JincResize::resize_plane_c<T,thr,subsampled> inner loops (src/JincResize.cpp:560-587) and its
  * SIMD siblings (src/resize_plane_{sse41,avx2,avx512}.cpp) for ONE plane.
- * sample_bytes: 1 (uint8), 2 (uint16, 10..16 bit) or 4 (float).  peak: (1<<bits)-1 for integer samples
- * (clamp + round-half-even, :581-582); ignored for float (:583-584).
+ * sample_bytes: 1 (uint8), 2 (uint16, 10..16 bit), 4 (float) or JINC_SAMPLE_F16 (half).  peak: (1<<bits)-1 for
+ * integer samples (clamp + round-half-even, :581-582); ignored for float and half (:583-584).
  * d_src/d_dst are device pointers, pitches in bytes; `stream` is a cudaStream_t (NULL = the context's
  * own stream).  Asynchronous with respect to the host.                                            */
 JINC_API int jinc_resize_plane_device(jinc_ctx* ctx, const jinc_table* t, int sample_bytes, float peak,
@@ -154,8 +162,8 @@ typedef struct jinc_filter_params {
     int32_t cplace;             /* JINC_CPLACE_* (used only when chroma is subsampled) */
     int32_t n_planes;           /* 1..4, processing order Y,U,V,A or G,B,R,A (:539-540) */
     int32_t sub_w, sub_h;       /* log2 chroma subsampling of planes 1,2 (0,0 for Y/444/RGB) */
-    int32_t sample_bytes;       /* 1, 2, 4 */
-    int32_t bits;               /* bits per component (8..16, 32) -> peak (:793) */
+    int32_t sample_bytes;       /* 1, 2, 4 or JINC_SAMPLE_F16 */
+    int32_t bits;               /* bits per component (8..16, 32; 16 for JINC_SAMPLE_F16) -> peak (:793) */
     int32_t n_devices;          /* 0 => all visible devices */
     int32_t devices[JINC_MAX_DEVICES];
     int32_t slots_per_device;   /* frames in flight per GPU (0 => 3..8, by frame size) */

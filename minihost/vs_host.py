@@ -41,6 +41,7 @@ def lib():
         L.vsmh_map_set_data.argtypes = [vp, C.c_char_p, C.c_char_p]
         L.vsmh_invoke.restype, L.vsmh_invoke.argtypes = vp, [vp, C.c_char_p, vp, C.c_char_p, ci]
         L.vsmh_node_info.argtypes = [vp] + [C.POINTER(ci)] * 5
+        L.vsmh_node_format.argtypes = [vp, C.POINTER(ci), C.POINTER(ci)]
         L.vsmh_get_frame.restype, L.vsmh_get_frame.argtypes = vp, [vp, ci, C.c_char_p, ci]
         L.vsmh_frame_plane.argtypes = [vp, ci, C.POINTER(vp), C.POINTER(C.c_ssize_t), C.POINTER(ci), C.POINTER(ci)]
         L.vsmh_frame_prop_int.restype, L.vsmh_frame_prop_int.argtypes = ci, [vp, C.c_char_p, C.POINTER(C.c_int64)]
@@ -66,6 +67,13 @@ class Node:
         v = [C.c_int() for _ in range(5)]
         lib().vsmh_node_info(self.handle, *[C.byref(x) for x in v])
         return dict(zip(("width", "height", "num_frames", "num_planes", "bytes_per_sample"), (x.value for x in v)))
+
+    @property
+    def format(self):
+        """(sample type, bits per sample) of the clip: ST_INT or ST_FLOAT."""
+        st, bits = C.c_int(), C.c_int()
+        lib().vsmh_node_format(self.handle, C.byref(st), C.byref(bits))
+        return st.value, bits.value
 
     def get_frame(self, n: int):
         """(planes, props): planes in VapourSynth order (Y,U,V or R,G,B)."""
@@ -115,7 +123,7 @@ class Core:
 
     def source(self, family: int, dtype, bits: int, ssw: int, ssh: int, width: int, height: int, frames, num_frames=None, props=None) -> Node:
         """frames: list (one per stored frame) of lists of 2-D numpy planes in VapourSynth order."""
-        st = ST_FLOAT if np.dtype(dtype) == np.float32 else ST_INT
+        st = ST_FLOAT if np.issubdtype(np.dtype(dtype), np.floating) else ST_INT
         h = lib().vsmh_source_create(self.handle, family, st, bits, ssw, ssh, width, height, num_frames or len(frames), len(frames))
         for k, planes in enumerate(frames):
             for p, arr in enumerate(planes):

@@ -585,6 +585,11 @@ VSMH_API void vsmh_node_info(VSNode* n, int* width, int* height, int* num_frames
     *num_planes = n->vi.format.numPlanes;
     *bytes_per_sample = n->vi.format.bytesPerSample;
 }
+VSMH_API void vsmh_node_format(VSNode* n, int* sample_type, int* bits_per_sample)
+{
+    *sample_type = n->vi.format.sampleType;
+    *bits_per_sample = n->vi.format.bitsPerSample;
+}
 VSMH_API const VSFrame* vsmh_get_frame(VSNode* n, int k, char* err, int err_size) { return api_get_frame(k, n, err, err_size); }
 VSMH_API void vsmh_frame_plane(const VSFrame* f, int plane, const uint8_t** ptr, ptrdiff_t* stride, int* w, int* h)
 {
