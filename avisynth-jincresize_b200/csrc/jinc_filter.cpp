@@ -127,6 +127,7 @@ struct Slot {
     uint32_t probe_seed = 0;
     bool probe_active = false;
     int src_row0[JINC_MAX_PLANES] = {}, src_row1[JINC_MAX_PLANES] = {}; // source rows uploaded per plane
+    float antiring = 0.f; // anti-ringing strength of the pending frame (captured when it was submitted)
 };
 
 constexpr int kRedoStaged = 1; // finish_frame: a registration turned out stale -- run the frame again through the mirrors
@@ -184,6 +185,7 @@ struct jinc_filter {
     int64_t next_ticket = 0; // under mu
     std::atomic<int64_t> rr{0};
     std::atomic<int64_t> launches{0};
+    std::atomic<float> antiring{0.f}; // jinc_filter_set_antiring; each frame reads it once, when it is submitted
     bool registers = false; // counted as a client of the host-buffer registry
 };
 
@@ -291,9 +293,11 @@ bool plane_range(const void* base, ptrdiff_t pitch, size_t row_bytes, int rows, 
     return true;
 }
 
-// Enqueue H2D + kernels + D2H for output rows [y0,y1) (luma rows) of `frame` on slot s.  staged_only: do not address the
-// caller's memory by DMA at all (the retry after a stale registration was found).
-int enqueue_frame(jinc_filter* f, Slot* s, const jinc_frame* frame, int y0_luma, int y1_luma, bool whole, bool staged_only = false)
+// Enqueue H2D + kernels + D2H for output rows [y0,y1) (luma rows) of `frame` on slot s, with anti-ringing strength
+// `antiring` (0: off).  staged_only: do not address the caller's memory by DMA at all (the retry after a stale registration
+// was found).
+int enqueue_frame(jinc_filter* f, Slot* s, const jinc_frame* frame, int y0_luma, int y1_luma, bool whole, float antiring,
+                  bool staged_only = false)
 {
     DeviceState& d = f->devs[s->dev_index];
     JINC_CUDA(cudaSetDevice(d.ctx->device));
@@ -303,6 +307,7 @@ int enqueue_frame(jinc_filter* f, Slot* s, const jinc_frame* frame, int y0_luma,
     s->probe_active = false;
     const bool padding_ok = (f->p.flags & JINC_FILTER_DST_PADDING_WRITABLE) != 0;
     s->pending = *frame;
+    s->antiring = antiring;
     s->n_sentinels = 0;
 
     // per plane: the output rows of this band and the source rows its windows reach
@@ -476,8 +481,10 @@ int enqueue_frame(jinc_filter* f, Slot* s, const jinc_frame* frame, int y0_luma,
         if (n == 0)
             continue;
         int launched = 0;
-        const int rc = jinc_launch_resize_planes(d.ctx, d.tables[k], f->p.sample_bytes, f->peak, n, src, sp, dst, dp, yb, ye, s->stream,
-                                                  &launched);
+        int rc = jinc_launch_resize_planes(d.ctx, d.tables[k], f->p.sample_bytes, f->peak, n, src, sp, dst, dp, yb, ye, s->stream,
+                                            &launched);
+        if (rc == JINC_OK && antiring > 0.f)
+            rc = jinc_launch_antiring_planes(d.tables[k], f->p.sample_bytes, antiring, n, src, sp, dst, dp, yb, ye, s->stream, &launched);
         f->launches.fetch_add(launched);
         if (rc != JINC_OK)
             return rc;
@@ -620,7 +627,7 @@ int complete_frame(jinc_filter* f, Slot* s, int y0_luma, int y1_luma, bool whole
     const jinc_frame frame = s->pending;
     jinc_hostmem::release(&s->src_pin);
     jinc_hostmem::release(&s->dst_pin);
-    rc = enqueue_frame(f, s, &frame, y0_luma, y1_luma, whole, true);
+    rc = enqueue_frame(f, s, &frame, y0_luma, y1_luma, whole, s->antiring, true);
     if (rc != JINC_OK) {
         cudaStreamSynchronize(s->stream);
         return rc;
@@ -644,11 +651,12 @@ int submit_impl(jinc_filter* f, const jinc_frame* frame, int64_t* ticket, bool b
         return rc;
     if (!ticket)
         return jinc_fail(JINC_E_INVALID, "jinc_filter_submit: null ticket");
+    const float antiring = f->antiring.load();
     Slot* s = acquire_slot(f, block);
     if (!s)
         return jinc_fail(JINC_E_BUSY, "jinc_filter_try_submit: all %zu in-flight slots are taken", f->slots.size());
     const int64_t tk = s->ticket;
-    const int rc = enqueue_frame(f, s, frame, 0, f->p.target_h, true);
+    const int rc = enqueue_frame(f, s, frame, 0, f->p.target_h, true, antiring);
     if (rc != JINC_OK) {
         cudaStreamSynchronize(s->stream);
         release_slot(f, s);
@@ -825,6 +833,16 @@ extern "C" int jinc_filter_num_devices(const jinc_filter* f) { return f ? static
 extern "C" int jinc_filter_num_slots(const jinc_filter* f) { return f ? static_cast<int>(f->slots.size()) : 0; }
 extern "C" int64_t jinc_filter_kernel_launches(const jinc_filter* f) { return f ? f->launches.load() : 0; }
 
+extern "C" int jinc_filter_set_antiring(jinc_filter* f, float strength)
+{
+    if (!f)
+        return jinc_fail(JINC_E_INVALID, "jinc_filter_set_antiring: null filter");
+    if (!(strength >= 0.f && strength <= 1.f))
+        return jinc_fail(JINC_E_INVALID, "jinc_filter_set_antiring: strength must be between 0.0 and 1.0");
+    f->antiring.store(strength);
+    return JINC_OK;
+}
+
 extern "C" void jinc_host_buffer_stats(int64_t* registered_bytes, int64_t* registrations, int64_t* direct_src_frames,
                                        int64_t* direct_dst_frames, int64_t* staged_frames)
 {
@@ -844,8 +862,9 @@ extern "C" int jinc_filter_process(jinc_filter* f, const jinc_frame* frame)
 {
     if (int rc = check_frame(f, frame))
         return rc;
+    const float antiring = f->antiring.load();
     Slot* s = acquire_slot(f, true);
-    int rc = enqueue_frame(f, s, frame, 0, f->p.target_h, true);
+    int rc = enqueue_frame(f, s, frame, 0, f->p.target_h, true, antiring);
     if (rc == JINC_OK)
         rc = complete_frame(f, s, 0, f->p.target_h, true);
     else
@@ -864,6 +883,7 @@ extern "C" int jinc_filter_process_device(jinc_filter* f, int device_index, cons
     DeviceState& d = f->devs[device_index];
     JINC_CUDA(cudaSetDevice(d.ctx->device));
     cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d.ctx->stream;
+    const float antiring = f->antiring.load();
     for (int k = 0; k < f->n_tables; ++k) {
         if (!(table_mask & (1 << k)))
             continue;
@@ -883,8 +903,11 @@ extern "C" int jinc_filter_process_device(jinc_filter* f, int device_index, cons
         if (n == 0)
             continue;
         int launched = 0;
-        const int rc = jinc_launch_resize_planes(d.ctx, d.tables[k], f->p.sample_bytes, f->peak, n, src, sp, dst, dp, 0,
-                                                 d.tables[k]->sc.dst_h, st, &launched, parts);
+        int rc = jinc_launch_resize_planes(d.ctx, d.tables[k], f->p.sample_bytes, f->peak, n, src, sp, dst, dp, 0,
+                                           d.tables[k]->sc.dst_h, st, &launched, parts);
+        if (rc == JINC_OK && antiring > 0.f && parts == JINC_PART_ALL)
+            rc = jinc_launch_antiring_planes(d.tables[k], f->p.sample_bytes, antiring, n, src, sp, dst, dp, 0, d.tables[k]->sc.dst_h, st,
+                                             &launched);
         f->launches.fetch_add(launched);
         if (rc != JINC_OK)
             return rc;
@@ -902,6 +925,7 @@ extern "C" int jinc_filter_process_device_batch(jinc_filter* f, int device_index
     DeviceState& d = f->devs[device_index];
     JINC_CUDA(cudaSetDevice(d.ctx->device));
     cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d.ctx->stream;
+    const float antiring = f->antiring.load();
     const size_t rec = jinc_plane_ptrs_size();
     for (int k = 0; k < f->n_tables; ++k) {
         if (!(table_mask & (1 << k)))
@@ -953,7 +977,9 @@ extern "C" int jinc_filter_process_device_batch(jinc_filter* f, int device_index
         // pageable source: staged by the runtime before the call returns, ordered before the kernel on `st`
         JINC_CUDA(cudaMemcpyAsync(dbuf, host.data(), host.size(), cudaMemcpyHostToDevice, st));
         int launched = 0;
-        const int rc = jinc_launch_resize_batch(d.ctx, d.tables[k], f->p.sample_bytes, f->peak, n, dbuf, n_frames, st, &launched, parts);
+        int rc = jinc_launch_resize_batch(d.ctx, d.tables[k], f->p.sample_bytes, f->peak, n, dbuf, n_frames, st, &launched, parts);
+        if (rc == JINC_OK && antiring > 0.f && parts == JINC_PART_ALL) // before the record: the pass reads the same plane-pointer records
+            rc = jinc_launch_antiring_batch(d.tables[k], f->p.sample_bytes, antiring, n, dbuf, n_frames, st, &launched);
         f->launches.fetch_add(launched);
         JINC_CUDA(cudaEventRecord(d.batch_done[slot], st));
         if (rc != JINC_OK)
@@ -1022,6 +1048,7 @@ extern "C" int jinc_filter_process_bands(jinc_filter* f, const jinc_frame* frame
     std::vector<int32_t> yb(n_bands), ye(n_bands);
     if (int rc = jinc_plan_row_bands(f->p.target_h, n_bands, yb.data(), ye.data()))
         return rc;
+    const float antiring = f->antiring.load(); // one strength for every band of the frame
 
     // Band i runs on GPU i % G through a slot of that GPU.  This caller never blocks on a slot while it holds one: when
     // its GPU has none free it first completes its own oldest band, so concurrent callers cannot deadlock each other.
@@ -1065,7 +1092,7 @@ extern "C" int jinc_filter_process_bands(jinc_filter* f, const jinc_frame* frame
         }
         if (!s)
             break;
-        rc = enqueue_frame(f, s, frame, yb[i], ye[i], false);
+        rc = enqueue_frame(f, s, frame, yb[i], ye[i], false, antiring);
         if (rc != JINC_OK) {
             cudaStreamSynchronize(s->stream);
             release_slot(f, s);

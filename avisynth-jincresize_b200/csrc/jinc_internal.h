@@ -227,6 +227,14 @@ int jinc_pack_plane_ptrs(void* out, int sample, int n_planes, const void* const*
                          void* const* d_dst, const ptrdiff_t* dst_pitch);
 int jinc_launch_resize_batch(jinc_ctx* ctx, const jinc_table* t, int sample, float peak, int n_planes,
                              const void* d_frame_ptrs, int n_frames, cudaStream_t stream, int* launches, int parts);
+// jinc_antiring.cu: the anti-ringing clamp in place on planes the two launchers above produced, with the same plane
+// arguments (rows [y_begin,y_end) read the same source rows as the resample launch of that band).  strength in [0, 1];
+// 0 launches nothing.  Needs complete output samples: run it after a JINC_PART_ALL resample launch.
+int jinc_launch_antiring_planes(const jinc_table* t, int sample, float strength, int n_planes, const void* const* d_src,
+                                const ptrdiff_t* src_pitch, void* const* d_dst, const ptrdiff_t* dst_pitch, int y_begin,
+                                int y_end, cudaStream_t stream, int* launches);
+int jinc_launch_antiring_batch(const jinc_table* t, int sample, float strength, int n_planes, const void* d_frame_ptrs,
+                               int n_frames, cudaStream_t stream, int* launches);
 int jinc_debug_pixel_weights(const jinc_table* t, int x, int y, float* out);
 // probe words of a device buffer: d_out[k] = 32-bit word jinc_probe_index(seed, k, n_words) of d_buf, k < JINC_PROBE_WORDS
 constexpr int JINC_PROBE_WORDS = 256;

@@ -67,7 +67,8 @@ EXPORTS = [
     "jinc_filter_process", "jinc_filter_submit", "jinc_filter_wait", "jinc_filter_process_split",
     "jinc_filter_kernel_launches", "jinc_filter_process_device", "jinc_filter_process_device_batch",
     "jinc_plan_frame_owner", "jinc_plan_row_bands", "jinc_filter_num_slots", "jinc_filter_try_submit",
-    "jinc_filter_process_bands", "jinc_host_buffer_stats", "jinc_filter_live_count",
+    "jinc_filter_process_bands", "jinc_host_buffer_stats", "jinc_filter_live_count", "jinc_filter_set_antiring",
+    "jinc_antiring_plane_device",
 ]
 
 _lib = None
@@ -99,6 +100,9 @@ def lib():
         L.jinc_table_pixel_block.restype, L.jinc_table_pixel_block.argtypes = ci, [vp, ci, ci, C.POINTER(C.c_int64)]
         L.jinc_resize_plane_device.restype = ci
         L.jinc_resize_plane_device.argtypes = [vp, vp, ci, C.c_float, vp, C.c_ssize_t, vp, C.c_ssize_t, vp]
+        L.jinc_antiring_plane_device.restype = ci
+        L.jinc_antiring_plane_device.argtypes = [vp, vp, ci, C.c_float, vp, C.c_ssize_t, vp, C.c_ssize_t, vp]
+        L.jinc_filter_set_antiring.restype, L.jinc_filter_set_antiring.argtypes = ci, [vp, C.c_float]
         L.jinc_table_launches_per_plane.restype, L.jinc_table_launches_per_plane.argtypes = ci, [vp]
         L.jinc_table_strip_plan.restype, L.jinc_table_strip_plan.argtypes = ci, [vp, C.POINTER(ci)]
         L.jinc_filter_create.restype, L.jinc_filter_create.argtypes = ci, [C.POINTER(FilterParams), C.POINTER(vp)]
@@ -260,6 +264,12 @@ class Table(TableView):
         _check(lib().jinc_resize_plane_device(self.ctx.handle, self.handle, sample_bytes, peak, d_src, src_pitch,
                                               d_dst, dst_pitch, stream or None))
 
+    def antiring_device(self, sample_bytes: int, strength: float, d_src: int, src_pitch: int, d_dst: int, dst_pitch: int,
+                        stream: int = 0):
+        """Anti-ringing clamp in place on a plane resize_device produced from d_src (jinc_antiring_plane_device)."""
+        _check(lib().jinc_antiring_plane_device(self.ctx.handle, self.handle, sample_bytes, strength, d_src, src_pitch,
+                                                d_dst, dst_pitch, stream or None))
+
     def close(self):
         if self.handle:
             lib().jinc_table_destroy(self.handle)
@@ -332,6 +342,10 @@ class Filter:
     @property
     def kernel_launches(self) -> int:
         return lib().jinc_filter_kernel_launches(self.handle)
+
+    def set_antiring(self, strength: float):
+        """Anti-ringing strength of frames submitted from now on: 0 (off, the default) .. 1 (jinc_filter_set_antiring)."""
+        _check(lib().jinc_filter_set_antiring(self.handle, strength))
 
     def _frame(self, src_planes, dst_planes) -> Frame:
         fr = Frame()

@@ -140,6 +140,19 @@ JINC_API int jinc_resize_plane_device(jinc_ctx* ctx, const jinc_table* t, int sa
                                       void* stream);
 /* number of kernel launches the call above issues for this table (fast-path interior + border strips) */
 JINC_API int jinc_table_launches_per_plane(const jinc_table* t);
+/* Anti-ringing clamp, in place, on a plane that jinc_resize_plane_device produced from d_src with the same table (no
+ * reference counterpart: the reference has no anti-ringing).  Every output sample y is pulled toward the range [lo, hi]
+ * of the 2x2 source samples around its position: with pos_x / pos_y the table's accumulated positions (jinc_table_axis),
+ * ax0 = clamp(floor(pos_x), 0, src_w-1), ax1 = clamp(floor(pos_x)+1, 0, src_w-1), ay0 / ay1 likewise; lo / hi are fminf /
+ * fmaxf over src[ay0|ay1][ax0|ax1] (NaN samples ignored); c = fminf(fmaxf(y, lo), hi); the result is c when
+ * strength == 1, else fmaf(strength, c, (1 - strength) * y) in float, and y itself when y is NaN.  Integer samples are
+ * rounded half to even, half samples to the nearest half.  At strength 1 every output lies in [lo, hi] (a +-Inf output
+ * becomes the bound); below 1 a +-Inf output stays +-Inf.  strength: 0..1, 0 = off (a valid call that launches nothing).
+ * Same sample_bytes, pitch and alignment rules (destination 16-byte aligned, pitch multiple of 16) and stream semantics as
+ * jinc_resize_plane_device.                                                                      */
+JINC_API int jinc_antiring_plane_device(jinc_ctx* ctx, const jinc_table* t, int sample_bytes, float strength,
+                                        const void* d_src, ptrdiff_t src_pitch, void* d_dst, ptrdiff_t dst_pitch,
+                                        void* stream);
 /* Introspection of the table's strip plan (no reference counterpart: the reference keeps one weight block per border
  * pixel, src/JincResize.cpp:443-518, and has no notion of patches).  Whole-frame launches of the exact-2x, chunked-cells
  * and integer-ratio kernels run their border strips from descriptors worked out once per table; returns the number of
@@ -247,6 +260,14 @@ JINC_API int jinc_filter_process_device(jinc_filter* f, int device_index, const 
  * has finished. */
 JINC_API int jinc_filter_process_device_batch(jinc_filter* f, int device_index, const jinc_frame* frames, int n_frames,
                                               int table_mask, int parts, void* stream);
+/* Anti-ringing strength of the filter (no reference counterpart): 0 (the default) = off, 1 = every output sample clamped
+ * to the range of the 2x2 source samples around it, in between a blend (see jinc_antiring_plane_device for the exact
+ * definition).  When it is > 0, each resample launch of a frame is followed by one anti-ringing launch on the same stream,
+ * before the copy back; jinc_filter_process_device(_batch) run it only with parts = JINC_PART_ALL.  Thread-safe; a frame
+ * uses the strength current when it is submitted (jinc_filter_process, _submit, _try_submit, _process_bands / _split, the
+ * device calls), so it applies to frames submitted after this call returns.  JINC_E_INVALID for a NULL filter or a
+ * strength that is NaN or outside [0, 1]. */
+JINC_API int jinc_filter_set_antiring(jinc_filter* f, float strength);
 /* kernels launched so far by this filter (all devices) */
 JINC_API int64_t jinc_filter_kernel_launches(const jinc_filter* f);
 /* host-buffer bookkeeping of the frame pipeline (process-wide): bytes of caller memory currently page-locked by
