@@ -65,11 +65,53 @@ extern "C" int jinc_ctx_create(int device, jinc_ctx** out)
     return JINC_OK;
 }
 
+int jinc_ring_launch(jinc_ctx* ctx, const void* host, size_t bytes, cudaStream_t st, const std::function<int(const void*)>& launch)
+{
+    RecordRing& r = ctx->ring;
+    std::lock_guard<std::mutex> lk(r.mu);
+    const int slot = r.next;
+    r.next = (r.next + 1) % RecordRing::kRing;
+    if (!r.done[slot])
+        JINC_CUDA(cudaEventCreateWithFlags(&r.done[slot], cudaEventDisableTiming));
+    else
+        JINC_CUDA(cudaStreamWaitEvent(st, r.done[slot], 0)); // the launch that last read this entry
+    if (r.cap[slot] < bytes) {
+        JINC_CUDA(cudaEventSynchronize(r.done[slot])); // no-op for a fresh event
+        cudaFree(r.ptrs[slot]);
+        r.ptrs[slot] = nullptr;
+        r.cap[slot] = 0;
+        if (cudaMalloc(reinterpret_cast<void**>(&r.ptrs[slot]), bytes) != cudaSuccess)
+            return jinc_fail(JINC_E_NOMEM, "plane records: cudaMalloc(%zu) failed", bytes);
+        r.cap[slot] = bytes;
+    }
+    // pageable source: staged by the runtime before the call returns, ordered before the kernel on `st`
+    JINC_CUDA(cudaMemcpyAsync(r.ptrs[slot], host, bytes, cudaMemcpyHostToDevice, st));
+    const int rc = launch(r.ptrs[slot]);
+    JINC_CUDA(cudaEventRecord(r.done[slot], st));
+    return rc;
+}
+
+void jinc_ring_free(jinc_ctx* ctx)
+{
+    RecordRing& r = ctx->ring;
+    for (int k = 0; k < RecordRing::kRing; ++k) {
+        if (r.done[k]) {
+            cudaEventSynchronize(r.done[k]);
+            cudaEventDestroy(r.done[k]);
+            r.done[k] = nullptr;
+        }
+        cudaFree(r.ptrs[k]);
+        r.ptrs[k] = nullptr;
+        r.cap[k] = 0;
+    }
+}
+
 extern "C" void jinc_ctx_destroy(jinc_ctx* ctx)
 {
     if (!ctx)
         return;
     cudaSetDevice(ctx->device);
+    jinc_ring_free(ctx);
     if (ctx->stream)
         cudaStreamDestroy(ctx->stream);
     delete ctx;
@@ -135,13 +177,6 @@ constexpr int kRedoStaged = 1; // finish_frame: a registration turned out stale 
 struct DeviceState {
     jinc_ctx* ctx = nullptr;
     jinc_table* tables[2] = {nullptr, nullptr};
-    // ring of small device buffers holding the plane-pointer records of batched launches; an entry is reused only after
-    // the launch that read it has finished (event), whatever streams the calls use
-    static constexpr int kRing = 8;
-    unsigned char* batch_ptrs[kRing] = {};
-    size_t batch_cap[kRing] = {};
-    cudaEvent_t batch_done[kRing] = {};
-    int batch_next = 0;
 };
 
 // rows of one plane between host and device.  `linear`: both sides have the same pitch and the bytes between rows may be
@@ -690,14 +725,9 @@ extern "C" void jinc_filter_destroy(jinc_filter* f)
             cudaStreamDestroy(s->stream);
     }
     for (DeviceState& d : f->devs) {
-        if (d.ctx)
+        if (d.ctx) {
             cudaSetDevice(d.ctx->device);
-        for (int k = 0; k < DeviceState::kRing; ++k) {
-            if (d.batch_done[k]) {
-                cudaEventSynchronize(d.batch_done[k]);
-                cudaEventDestroy(d.batch_done[k]);
-            }
-            cudaFree(d.batch_ptrs[k]);
+            jinc_ring_free(d.ctx); // batched launches still reading the tables finish first
         }
         jinc_table_destroy(d.tables[0]);
         jinc_table_destroy(d.tables[1]);
@@ -955,33 +985,14 @@ extern "C" int jinc_filter_process_device_batch(jinc_filter* f, int device_index
         }
         if (n == 0)
             continue;
-        // The whole sequence -- take the ring entry, order it after its previous reader, upload, launch, record -- runs
-        // under the lock, so two callers on different streams cannot interleave on one entry.
-        std::lock_guard<std::mutex> lk(f->mu);
-        const int slot = d.batch_next;
-        d.batch_next = (d.batch_next + 1) % DeviceState::kRing;
-        if (!d.batch_done[slot])
-            JINC_CUDA(cudaEventCreateWithFlags(&d.batch_done[slot], cudaEventDisableTiming));
-        else
-            JINC_CUDA(cudaStreamWaitEvent(st, d.batch_done[slot], 0)); // the launch that last read this entry
-        if (d.batch_cap[slot] < host.size()) {
-            JINC_CUDA(cudaEventSynchronize(d.batch_done[slot])); // no-op for a fresh event
-            cudaFree(d.batch_ptrs[slot]);
-            d.batch_ptrs[slot] = nullptr;
-            d.batch_cap[slot] = 0;
-            if (cudaMalloc(reinterpret_cast<void**>(&d.batch_ptrs[slot]), host.size()) != cudaSuccess)
-                return jinc_fail(JINC_E_NOMEM, "jinc_filter_process_device_batch: cudaMalloc(%zu) failed", host.size());
-            d.batch_cap[slot] = host.size();
-        }
-        unsigned char* dbuf = d.batch_ptrs[slot];
-        // pageable source: staged by the runtime before the call returns, ordered before the kernel on `st`
-        JINC_CUDA(cudaMemcpyAsync(dbuf, host.data(), host.size(), cudaMemcpyHostToDevice, st));
         int launched = 0;
-        int rc = jinc_launch_resize_batch(d.ctx, d.tables[k], f->p.sample_bytes, f->peak, n, dbuf, n_frames, st, &launched, parts);
-        if (rc == JINC_OK && antiring > 0.f && parts == JINC_PART_ALL) // before the record: the pass reads the same plane-pointer records
-            rc = jinc_launch_antiring_batch(d.tables[k], f->p.sample_bytes, antiring, n, dbuf, n_frames, st, &launched);
+        const int rc = jinc_ring_launch(d.ctx, host.data(), host.size(), st, [&](const void* dbuf) {
+            int r = jinc_launch_resize_batch(d.ctx, d.tables[k], f->p.sample_bytes, f->peak, n, dbuf, n_frames, st, &launched, parts);
+            if (r == JINC_OK && antiring > 0.f && parts == JINC_PART_ALL) // before the record: the pass reads the same plane-pointer records
+                r = jinc_launch_antiring_batch(d.tables[k], f->p.sample_bytes, antiring, n, dbuf, n_frames, st, &launched);
+            return r;
+        });
         f->launches.fetch_add(launched);
-        JINC_CUDA(cudaEventRecord(d.batch_done[slot], st));
         if (rc != JINC_OK)
             return rc;
     }

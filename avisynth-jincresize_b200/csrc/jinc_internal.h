@@ -6,6 +6,8 @@
 
 #include <cstdarg>
 #include <cstdint>
+#include <functional>
+#include <mutex>
 #include <string>
 #include <vector>
 
@@ -27,12 +29,30 @@ int jinc_fail(int code, const char* fmt, ...) __attribute__((format(printf, 2, 3
     } while (0)
 
 // ---------------------------------------------------------------- context
+// Ring of small device buffers holding the plane-pointer records of batched launches.  An entry is reused only after the
+// launch that read it has finished (event), whatever streams the calls use.
+struct RecordRing {
+    static constexpr int kRing = 8;
+    std::mutex mu;
+    unsigned char* ptrs[kRing] = {};
+    size_t cap[kRing] = {};
+    cudaEvent_t done[kRing] = {};
+    int next = 0;
+};
+
 struct jinc_ctx {
     int device = -1;
     int sm_count = 0;
     size_t smem_optin = 0;
     cudaStream_t stream = nullptr; // default stream for table builds and callers that pass none
+    RecordRing ring;
 };
+
+// Uploads `bytes` of host records into the next entry of the context's ring on `st`, calls launch(device copy) and records
+// the entry's event after it.  The whole sequence runs under the ring's lock, so two callers on different streams cannot
+// interleave on one entry.  Returns launch's result, or the error of the upload.  Call with ctx->device current.
+int jinc_ring_launch(jinc_ctx* ctx, const void* host, size_t bytes, cudaStream_t st, const std::function<int(const void*)>& launch);
+void jinc_ring_free(jinc_ctx* ctx); // waits for the ring's last readers
 
 // ---------------------------------------------------------------- table
 // Geometry scalars of one table, derived on the host in the reference's own precision
@@ -235,6 +255,10 @@ int jinc_launch_antiring_planes(const jinc_table* t, int sample, float strength,
                                 int y_end, cudaStream_t stream, int* launches);
 int jinc_launch_antiring_batch(const jinc_table* t, int sample, float strength, int n_planes, const void* d_frame_ptrs,
                                int n_frames, cudaStream_t stream, int* launches);
+// jinc_adjoint.cu: the adjoint (jinc_b200.h, jinc_resize_adjoint_planes_device) of n_planes float planes; pitches and plane
+// strides in floats.  Adds the number of kernels launched to *launches.
+int jinc_launch_adjoint(const jinc_table* t, int n_planes, const float* g, long long g_pitch, long long g_stride, float* out,
+                        long long out_pitch, long long out_stride, cudaStream_t stream, int* launches);
 int jinc_debug_pixel_weights(const jinc_table* t, int x, int y, float* out);
 // probe words of a device buffer: d_out[k] = 32-bit word jinc_probe_index(seed, k, n_words) of d_buf, k < JINC_PROBE_WORDS
 constexpr int JINC_PROBE_WORDS = 256;

@@ -293,6 +293,8 @@ struct StripArgs {
 
 // whole-frame launches: the strip blocks of a table with a plan run from it (jinc_resize.cu)
 bool attach_strip_plan(const jinc_table* t, StripArgs& st, int threads, int spt);
+// the table's arrays and geometry scalars (no strips, no plan); jinc_resize.cu
+void fill_strip_args(const jinc_table* t, StripArgs& a);
 
 struct FrameSet {
     PlanePtrs one;           // used when frames == nullptr

@@ -242,7 +242,9 @@ __global__ void pixel_weights_kernel(StripArgs a, int x, int y, float* out)
     }
 }
 
-void fill_strip_args(const jinc_table* t, StripArgs& a)
+} // namespace
+
+void jinc_rs::fill_strip_args(const jinc_table* t, StripArgs& a)
 {
     memset(&a, 0, sizeof(a));
     a.start_x = t->ax[0].start;
@@ -268,6 +270,8 @@ void fill_strip_args(const jinc_table* t, StripArgs& a)
     a.radius2 = t->sc.radius2;
     a.idx_scale = t->sc.idx_scale;
 }
+
+namespace {
 
 // ------------------------------------------------------------------------------------------ launcher
 
@@ -1019,6 +1023,55 @@ extern "C" int jinc_resize_plane_device(jinc_ctx* ctx, const jinc_table* t, int 
     JINC_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
     return jinc_launch_resize(ctx, t, sample_bytes, peak, d_src, src_pitch, d_dst, dst_pitch, 0, t->sc.dst_h, st, nullptr);
+}
+
+extern "C" int jinc_resize_planes_device(jinc_ctx* ctx, const jinc_table* t, int sample_bytes, float peak, int n_planes,
+                                         const void* d_src, ptrdiff_t src_pitch, ptrdiff_t src_plane_stride, void* d_dst,
+                                         ptrdiff_t dst_pitch, ptrdiff_t dst_plane_stride, void* stream)
+{
+    if (!ctx || !t || !d_src || !d_dst)
+        return jinc_fail(JINC_E_INVALID, "jinc_resize_planes_device: null argument");
+    if (n_planes < 1)
+        return jinc_fail(JINC_E_INVALID, "jinc_resize_planes_device: n_planes must be at least 1");
+    if (!jinc_sample_valid(sample_bytes))
+        return jinc_fail(JINC_E_INVALID, "jinc_resize_planes_device: sample_bytes must be 1, 2, 4 or JINC_SAMPLE_F16");
+    if (reinterpret_cast<uintptr_t>(d_dst) % 16 || dst_pitch % 16 || (n_planes > 1 && dst_plane_stride % 16))
+        return jinc_fail(JINC_E_INVALID, "jinc_resize_planes_device: device destination planes must be 16-byte aligned (base, pitch and "
+                                         "plane stride)");
+    JINC_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    // records of up to four planes each (one block then serves the patch in all of them), grid.y = record
+    int per = JINC_MAX_PLANES;
+    while (n_planes % per)
+        --per;
+    const int n_rec = n_planes / per;
+    const size_t rec = sizeof(PlanePtrs);
+    constexpr int kMaxRecords = 65535; // grid.y limit
+    std::vector<unsigned char> host;
+    for (int r0 = 0; r0 < n_rec; r0 += kMaxRecords) {
+        const int nr = std::min(kMaxRecords, n_rec - r0);
+        host.assign(rec * nr, 0);
+        for (int r = 0; r < nr; ++r) {
+            const void* src[JINC_MAX_PLANES];
+            void* dst[JINC_MAX_PLANES];
+            ptrdiff_t sp[JINC_MAX_PLANES], dp[JINC_MAX_PLANES];
+            for (int k = 0; k < per; ++k) {
+                const long long i = (long long)(r0 + r) * per + k;
+                src[k] = static_cast<const unsigned char*>(d_src) + i * src_plane_stride;
+                dst[k] = static_cast<unsigned char*>(d_dst) + i * dst_plane_stride;
+                sp[k] = src_pitch;
+                dp[k] = dst_pitch;
+            }
+            if (int rc = jinc_pack_plane_ptrs(host.data() + rec * r, sample_bytes, per, src, sp, dst, dp))
+                return rc;
+        }
+        const int rc = jinc_ring_launch(ctx, host.data(), host.size(), st, [&](const void* dbuf) {
+            return jinc_launch_resize_batch(ctx, t, sample_bytes, peak, per, dbuf, nr, st, nullptr, JINC_PART_ALL);
+        });
+        if (rc != JINC_OK)
+            return rc;
+    }
+    return JINC_OK;
 }
 
 extern "C" int jinc_table_strip_plan(const jinc_table* t, int* staged)

@@ -68,7 +68,7 @@ EXPORTS = [
     "jinc_filter_kernel_launches", "jinc_filter_process_device", "jinc_filter_process_device_batch",
     "jinc_plan_frame_owner", "jinc_plan_row_bands", "jinc_filter_num_slots", "jinc_filter_try_submit",
     "jinc_filter_process_bands", "jinc_host_buffer_stats", "jinc_filter_live_count", "jinc_filter_set_antiring",
-    "jinc_antiring_plane_device",
+    "jinc_antiring_plane_device", "jinc_resize_planes_device", "jinc_resize_adjoint_planes_device",
 ]
 
 _lib = None
@@ -100,6 +100,11 @@ def lib():
         L.jinc_table_pixel_block.restype, L.jinc_table_pixel_block.argtypes = ci, [vp, ci, ci, C.POINTER(C.c_int64)]
         L.jinc_resize_plane_device.restype = ci
         L.jinc_resize_plane_device.argtypes = [vp, vp, ci, C.c_float, vp, C.c_ssize_t, vp, C.c_ssize_t, vp]
+        L.jinc_resize_planes_device.restype = ci
+        L.jinc_resize_planes_device.argtypes = [vp, vp, ci, C.c_float, ci, vp, C.c_ssize_t, C.c_ssize_t, vp, C.c_ssize_t,
+                                                C.c_ssize_t, vp]
+        L.jinc_resize_adjoint_planes_device.restype = ci
+        L.jinc_resize_adjoint_planes_device.argtypes = [vp, vp, ci, vp, C.c_ssize_t, C.c_ssize_t, vp, C.c_ssize_t, C.c_ssize_t, vp]
         L.jinc_antiring_plane_device.restype = ci
         L.jinc_antiring_plane_device.argtypes = [vp, vp, ci, C.c_float, vp, C.c_ssize_t, vp, C.c_ssize_t, vp]
         L.jinc_filter_set_antiring.restype, L.jinc_filter_set_antiring.argtypes = ci, [vp, C.c_float]
@@ -263,6 +268,20 @@ class Table(TableView):
         """One device-resident plane; sample_bytes is 1, 2, 4 or SAMPLE_F16 (peak is then ignored)."""
         _check(lib().jinc_resize_plane_device(self.ctx.handle, self.handle, sample_bytes, peak, d_src, src_pitch,
                                               d_dst, dst_pitch, stream or None))
+
+    def resize_planes_device(self, sample_bytes: int, peak: float, n_planes: int, d_src: int, src_pitch: int,
+                             src_plane_stride: int, d_dst: int, dst_pitch: int, dst_plane_stride: int, stream: int = 0):
+        """n_planes device-resident planes of this table's geometry in one call (jinc_resize_planes_device); pitches and
+        plane strides in bytes."""
+        _check(lib().jinc_resize_planes_device(self.ctx.handle, self.handle, sample_bytes, peak, n_planes, d_src, src_pitch,
+                                               src_plane_stride, d_dst, dst_pitch, dst_plane_stride, stream or None))
+
+    def adjoint_planes_device(self, n_planes: int, d_grad_dst: int, grad_dst_pitch: int, grad_dst_plane_stride: int,
+                              d_grad_src: int, grad_src_pitch: int, grad_src_plane_stride: int, stream: int = 0):
+        """Adjoint (transpose) of the resize on n_planes float32 gradient planes (jinc_resize_adjoint_planes_device)."""
+        _check(lib().jinc_resize_adjoint_planes_device(self.ctx.handle, self.handle, n_planes, d_grad_dst, grad_dst_pitch,
+                                                       grad_dst_plane_stride, d_grad_src, grad_src_pitch,
+                                                       grad_src_plane_stride, stream or None))
 
     def antiring_device(self, sample_bytes: int, strength: float, d_src: int, src_pitch: int, d_dst: int, dst_pitch: int,
                         stream: int = 0):

@@ -140,6 +140,34 @@ JINC_API int jinc_resize_plane_device(jinc_ctx* ctx, const jinc_table* t, int sa
                                       void* stream);
 /* number of kernel launches the call above issues for this table (fast-path interior + border strips) */
 JINC_API int jinc_table_launches_per_plane(const jinc_table* t);
+/* n_planes planes of one geometry; plane i at d_src + i*src_plane_stride / d_dst + i*dst_plane_stride (bytes).
+ * Byte-identical to n_planes calls of jinc_resize_plane_device; one launch per kernel for the whole batch (planes are grouped
+ * by up to four per record, in chunks of at most 65535 records).  Same sample_bytes, peak, pitch and alignment rules as
+ * jinc_resize_plane_device; the destination plane stride must also be a multiple of 16 when n_planes > 1.  The device
+ * array of plane records a launch reads comes from a small ring owned by ctx, whose entries are not reused before that
+ * launch has finished, so calls may use different streams.  Asynchronous on `stream` (NULL = the context's stream). */
+JINC_API int jinc_resize_planes_device(jinc_ctx* ctx, const jinc_table* t, int sample_bytes, float peak, int n_planes,
+                                       const void* d_src, ptrdiff_t src_pitch, ptrdiff_t src_plane_stride,
+                                       void* d_dst, ptrdiff_t dst_pitch, ptrdiff_t dst_plane_stride, void* stream);
+/* Adjoint of n_planes float32 gradient planes of the table's output size into float32 planes of its source size (no
+ * reference counterpart).  The resampler is a fixed linear map out = A * src; this computes A^T g:
+ *   grad_src[sy][sx] = sum over outputs (x, y) with start_x[x] <= sx < start_x[x]+fs and start_y[y] <= sy < start_y[y]+fs
+ *                      of w_{x,y}[sy - start_y[y]][sx - start_x[x]] * g[y][x]
+ * with start_x / start_y the window origins (jinc_table_axis) and w_{x,y} the weights of output (x, y)
+ * (jinc_table_pixel_weights), fs the filter size.
+ *  - Canonical order: output rows y ascending, within a row x ascending, acc = fmaf(w, g, acc) from 0.  Every kernel uses
+ *    it, so a source sample's bits do not depend on which kernel, tile, batch position or launch computed it.
+ *  - Every covering tap is multiplied, zero weights included: an Inf or NaN in g reaches every source sample of that
+ *    output's fs x fs window.
+ *  - Samples no output covers (outside a crop) are written as 0: every sample of grad_src is written, nothing accumulates.
+ *  - Gradients are float32 whatever the forward sample type; for integer planes this is the transpose of the linear map,
+ *    without the forward's rounding and clamping.
+ * 4-byte alignment and pitches only; pitches must hold a row and, when n_planes > 1, plane strides a plane.  d_grad_src
+ * must not overlap d_grad_dst.  Asynchronous on `stream` (NULL = the context's stream). */
+JINC_API int jinc_resize_adjoint_planes_device(jinc_ctx* ctx, const jinc_table* t, int n_planes,
+                                               const float* d_grad_dst, ptrdiff_t grad_dst_pitch, ptrdiff_t grad_dst_plane_stride,
+                                               float* d_grad_src, ptrdiff_t grad_src_pitch, ptrdiff_t grad_src_plane_stride,
+                                               void* stream);
 /* Anti-ringing clamp, in place, on a plane that jinc_resize_plane_device produced from d_src with the same table (no
  * reference counterpart: the reference has no anti-ringing).  Every output sample y is pulled toward the range [lo, hi]
  * of the 2x2 source samples around its position: with pos_x / pos_y the table's accumulated positions (jinc_table_axis),
