@@ -259,6 +259,26 @@ int jinc_launch_antiring_batch(const jinc_table* t, int sample, float strength, 
 // strides in floats.  Adds the number of kernels launched to *launches.
 int jinc_launch_adjoint(const jinc_table* t, int n_planes, const float* g, long long g_pitch, long long g_stride, float* out,
                         long long out_pitch, long long out_stride, cudaStream_t stream, int* launches);
+// jinc_antiring_adjoint.cu: the derivative of the anti-ringing clamp (jinc_b200.h, jinc_antiring_adjoint_planes_device).
+// Plane i of each array at base + i * stride; pitches and strides in elements (src / y: the forward's float or half samples).
+struct ArAdjPlanes {
+    const void* src;
+    long long src_pitch, src_stride;
+    const void* y; // the resized planes before the clamp
+    long long y_pitch, y_stride;
+    const float* g; // output gradient
+    long long g_pitch, g_stride;
+    float* gy; // written: gradient of the resized planes
+    long long gy_pitch, gy_stride;
+    float* gs; // written: source gradient
+    long long gs_pitch, gs_stride;
+    int n_planes;
+};
+// Three launches on `stream`: antiring_grad_out (g -> gy), jinc_launch_adjoint (gy -> gs), antiring_route_gather (gs += r);
+// at strength 0 a copy of g into gy and the plain adjoint.  sample 4 or JINC_SAMPLE_F16, strength in [0, 1].  Adds the
+// number of kernels launched to *launches.
+int jinc_launch_antiring_adjoint(const jinc_table* t, int sample, float strength, const ArAdjPlanes& p, cudaStream_t stream,
+                                 int* launches);
 int jinc_debug_pixel_weights(const jinc_table* t, int x, int y, float* out);
 // probe words of a device buffer: d_out[k] = 32-bit word jinc_probe_index(seed, k, n_words) of d_buf, k < JINC_PROBE_WORDS
 constexpr int JINC_PROBE_WORDS = 256;

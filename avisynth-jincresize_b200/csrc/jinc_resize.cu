@@ -1025,22 +1025,13 @@ extern "C" int jinc_resize_plane_device(jinc_ctx* ctx, const jinc_table* t, int 
     return jinc_launch_resize(ctx, t, sample_bytes, peak, d_src, src_pitch, d_dst, dst_pitch, 0, t->sc.dst_h, st, nullptr);
 }
 
-extern "C" int jinc_resize_planes_device(jinc_ctx* ctx, const jinc_table* t, int sample_bytes, float peak, int n_planes,
-                                         const void* d_src, ptrdiff_t src_pitch, ptrdiff_t src_plane_stride, void* d_dst,
-                                         ptrdiff_t dst_pitch, ptrdiff_t dst_plane_stride, void* stream)
+// n_planes planes of one geometry, plane i at d_src + i * src_plane_stride / d_dst + i * dst_plane_stride: grouped into
+// records of up to four planes (one block then serves its tile in all of them), in chunks of at most 65535 records (the
+// grid.y limit) uploaded through the context's ring; launch(device records, planes per record, records) enqueues a chunk.
+static int launch_plane_records(jinc_ctx* ctx, int sample, int n_planes, const void* d_src, ptrdiff_t src_pitch,
+                                ptrdiff_t src_plane_stride, void* d_dst, ptrdiff_t dst_pitch, ptrdiff_t dst_plane_stride,
+                                cudaStream_t st, const std::function<int(const void*, int, int)>& launch)
 {
-    if (!ctx || !t || !d_src || !d_dst)
-        return jinc_fail(JINC_E_INVALID, "jinc_resize_planes_device: null argument");
-    if (n_planes < 1)
-        return jinc_fail(JINC_E_INVALID, "jinc_resize_planes_device: n_planes must be at least 1");
-    if (!jinc_sample_valid(sample_bytes))
-        return jinc_fail(JINC_E_INVALID, "jinc_resize_planes_device: sample_bytes must be 1, 2, 4 or JINC_SAMPLE_F16");
-    if (reinterpret_cast<uintptr_t>(d_dst) % 16 || dst_pitch % 16 || (n_planes > 1 && dst_plane_stride % 16))
-        return jinc_fail(JINC_E_INVALID, "jinc_resize_planes_device: device destination planes must be 16-byte aligned (base, pitch and "
-                                         "plane stride)");
-    JINC_CUDA(cudaSetDevice(ctx->device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
-    // records of up to four planes each (one block then serves the patch in all of them), grid.y = record
     int per = JINC_MAX_PLANES;
     while (n_planes % per)
         --per;
@@ -1062,16 +1053,60 @@ extern "C" int jinc_resize_planes_device(jinc_ctx* ctx, const jinc_table* t, int
                 sp[k] = src_pitch;
                 dp[k] = dst_pitch;
             }
-            if (int rc = jinc_pack_plane_ptrs(host.data() + rec * r, sample_bytes, per, src, sp, dst, dp))
+            if (int rc = jinc_pack_plane_ptrs(host.data() + rec * r, sample, per, src, sp, dst, dp))
                 return rc;
         }
-        const int rc = jinc_ring_launch(ctx, host.data(), host.size(), st, [&](const void* dbuf) {
-            return jinc_launch_resize_batch(ctx, t, sample_bytes, peak, per, dbuf, nr, st, nullptr, JINC_PART_ALL);
-        });
+        const int rc = jinc_ring_launch(ctx, host.data(), host.size(), st, [&](const void* dbuf) { return launch(dbuf, per, nr); });
         if (rc != JINC_OK)
             return rc;
     }
     return JINC_OK;
+}
+
+extern "C" int jinc_resize_planes_device(jinc_ctx* ctx, const jinc_table* t, int sample_bytes, float peak, int n_planes,
+                                         const void* d_src, ptrdiff_t src_pitch, ptrdiff_t src_plane_stride, void* d_dst,
+                                         ptrdiff_t dst_pitch, ptrdiff_t dst_plane_stride, void* stream)
+{
+    if (!ctx || !t || !d_src || !d_dst)
+        return jinc_fail(JINC_E_INVALID, "jinc_resize_planes_device: null argument");
+    if (n_planes < 1)
+        return jinc_fail(JINC_E_INVALID, "jinc_resize_planes_device: n_planes must be at least 1");
+    if (!jinc_sample_valid(sample_bytes))
+        return jinc_fail(JINC_E_INVALID, "jinc_resize_planes_device: sample_bytes must be 1, 2, 4 or JINC_SAMPLE_F16");
+    if (reinterpret_cast<uintptr_t>(d_dst) % 16 || dst_pitch % 16 || (n_planes > 1 && dst_plane_stride % 16))
+        return jinc_fail(JINC_E_INVALID, "jinc_resize_planes_device: device destination planes must be 16-byte aligned (base, pitch and "
+                                         "plane stride)");
+    JINC_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    return launch_plane_records(ctx, sample_bytes, n_planes, d_src, src_pitch, src_plane_stride, d_dst, dst_pitch, dst_plane_stride, st,
+                                [&](const void* dbuf, int per, int nr) {
+                                    return jinc_launch_resize_batch(ctx, t, sample_bytes, peak, per, dbuf, nr, st, nullptr, JINC_PART_ALL);
+                                });
+}
+
+extern "C" int jinc_antiring_planes_device(jinc_ctx* ctx, const jinc_table* t, int sample_bytes, float strength, int n_planes,
+                                           const void* d_src, ptrdiff_t src_pitch, ptrdiff_t src_plane_stride, void* d_dst,
+                                           ptrdiff_t dst_pitch, ptrdiff_t dst_plane_stride, void* stream)
+{
+    if (!ctx || !t || !d_src || !d_dst)
+        return jinc_fail(JINC_E_INVALID, "jinc_antiring_planes_device: null argument");
+    if (n_planes < 1)
+        return jinc_fail(JINC_E_INVALID, "jinc_antiring_planes_device: n_planes must be at least 1");
+    if (!jinc_sample_valid(sample_bytes))
+        return jinc_fail(JINC_E_INVALID, "jinc_antiring_planes_device: sample_bytes must be 1, 2, 4 or JINC_SAMPLE_F16");
+    if (!(strength >= 0.f && strength <= 1.f))
+        return jinc_fail(JINC_E_INVALID, "jinc_antiring_planes_device: strength must be between 0.0 and 1.0");
+    if (reinterpret_cast<uintptr_t>(d_dst) % 16 || dst_pitch % 16 || (n_planes > 1 && dst_plane_stride % 16))
+        return jinc_fail(JINC_E_INVALID, "jinc_antiring_planes_device: device destination planes must be 16-byte aligned (base, pitch "
+                                         "and plane stride)");
+    if (strength == 0.f)
+        return JINC_OK; // off: as jinc_antiring_plane_device, nothing is launched
+    JINC_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    return launch_plane_records(ctx, sample_bytes, n_planes, d_src, src_pitch, src_plane_stride, d_dst, dst_pitch, dst_plane_stride, st,
+                                [&](const void* dbuf, int per, int nr) {
+                                    return jinc_launch_antiring_batch(t, sample_bytes, strength, per, dbuf, nr, st, nullptr);
+                                });
 }
 
 extern "C" int jinc_table_strip_plan(const jinc_table* t, int* staged)

@@ -69,6 +69,7 @@ EXPORTS = [
     "jinc_plan_frame_owner", "jinc_plan_row_bands", "jinc_filter_num_slots", "jinc_filter_try_submit",
     "jinc_filter_process_bands", "jinc_host_buffer_stats", "jinc_filter_live_count", "jinc_filter_set_antiring",
     "jinc_antiring_plane_device", "jinc_resize_planes_device", "jinc_resize_adjoint_planes_device",
+    "jinc_antiring_planes_device", "jinc_antiring_adjoint_planes_device",
 ]
 
 _lib = None
@@ -105,6 +106,11 @@ def lib():
                                                 C.c_ssize_t, vp]
         L.jinc_resize_adjoint_planes_device.restype = ci
         L.jinc_resize_adjoint_planes_device.argtypes = [vp, vp, ci, vp, C.c_ssize_t, C.c_ssize_t, vp, C.c_ssize_t, C.c_ssize_t, vp]
+        L.jinc_antiring_planes_device.restype = ci
+        L.jinc_antiring_planes_device.argtypes = [vp, vp, ci, C.c_float, ci, vp, C.c_ssize_t, C.c_ssize_t, vp, C.c_ssize_t,
+                                                  C.c_ssize_t, vp]
+        L.jinc_antiring_adjoint_planes_device.restype = ci
+        L.jinc_antiring_adjoint_planes_device.argtypes = [vp, vp, ci, C.c_float, ci] + [vp, C.c_ssize_t, C.c_ssize_t] * 5 + [vp]
         L.jinc_antiring_plane_device.restype = ci
         L.jinc_antiring_plane_device.argtypes = [vp, vp, ci, C.c_float, vp, C.c_ssize_t, vp, C.c_ssize_t, vp]
         L.jinc_filter_set_antiring.restype, L.jinc_filter_set_antiring.argtypes = ci, [vp, C.c_float]
@@ -282,6 +288,21 @@ class Table(TableView):
         _check(lib().jinc_resize_adjoint_planes_device(self.ctx.handle, self.handle, n_planes, d_grad_dst, grad_dst_pitch,
                                                        grad_dst_plane_stride, d_grad_src, grad_src_pitch,
                                                        grad_src_plane_stride, stream or None))
+
+    def antiring_planes_device(self, sample_bytes: int, strength: float, n_planes: int, d_src: int, src_pitch: int,
+                               src_plane_stride: int, d_dst: int, dst_pitch: int, dst_plane_stride: int, stream: int = 0):
+        """Anti-ringing clamp in place on n_planes planes resize_planes_device produced (jinc_antiring_planes_device)."""
+        _check(lib().jinc_antiring_planes_device(self.ctx.handle, self.handle, sample_bytes, strength, n_planes, d_src,
+                                                 src_pitch, src_plane_stride, d_dst, dst_pitch, dst_plane_stride,
+                                                 stream or None))
+
+    def antiring_adjoint_planes_device(self, sample_bytes: int, strength: float, n_planes: int, src, y, grad_dst, grad_y,
+                                       grad_src, stream: int = 0):
+        """Gradient of resize + anti-ringing clamp (jinc_antiring_adjoint_planes_device) for float32 / SAMPLE_F16 planes.
+        src, y, grad_dst, grad_y, grad_src: (device pointer, pitch, plane stride) in bytes; writes grad_y and grad_src."""
+        planes = [v for t in (src, y, grad_dst, grad_y, grad_src) for v in t]
+        _check(lib().jinc_antiring_adjoint_planes_device(self.ctx.handle, self.handle, sample_bytes, strength, n_planes,
+                                                         *planes, stream or None))
 
     def antiring_device(self, sample_bytes: int, strength: float, d_src: int, src_pitch: int, d_dst: int, dst_pitch: int,
                         stream: int = 0):

@@ -9,6 +9,11 @@ out = A * src; for float16 and float32 inputs the op is a torch.autograd.Functio
 (jinc_resize_adjoint_planes_device) in float32 and casts the result to x.dtype.  There is no gradient with respect to the
 geometry arguments, and none for integer planes.
 
+antiring=s > 0 follows the resize with the anti-ringing clamp (jinc_antiring_planes_device), as the VapourSynth filter's
+`antiring` does.  The clamp is piecewise linear; for float16 / float32 inputs its backward recomputes the resized planes
+with one forward launch and runs jinc_antiring_adjoint_planes_device: the gradient of a clamped output goes, scaled by s,
+to the source sample that bounded it, the rest of it (1 - s) through the adjoint of the resize.
+
 Work runs on torch.cuda.current_stream(x.device) with no host synchronisation.  One library context is kept per device and
 a small LRU cache of coefficient tables keyed by (device, table parameters); building a table is synchronous, so a cached
 table is ready before any launch reads it.
@@ -35,7 +40,7 @@ def _f32(v) -> float:
     return float(np.float32(v))  # script floats are 32-bit
 
 
-def _check_args(x, width, height, tap, quant_x, quant_y, bits) -> int:
+def _check_args(x, width, height, tap, quant_x, quant_y, bits, antiring) -> int:
     """Validates everything that needs no GPU; returns the bits per sample (0 for float planes)."""
     if not isinstance(x, torch.Tensor):
         raise TypeError(f"jinc_resize: expected a torch.Tensor, got {type(x).__name__}")
@@ -53,6 +58,8 @@ def _check_args(x, width, height, tap, quant_x, quant_y, bits) -> int:
         if bits is not None:
             raise ValueError(f"jinc_resize: bits applies to integer planes only, got bits={bits} for {x.dtype}")
         bits = 0
+    if not (0.0 <= antiring <= 1.0):
+        raise ValueError("jinc_resize: antiring must be between 0.0 and 1.0.")
     if x.device.type != "cuda":
         raise ValueError(f"jinc_resize: x is on {x.device}; the resize has no CPU path, move the tensor to a CUDA device")
     if x.dim() < 2:
@@ -145,6 +152,16 @@ def _adjoint(grad: torch.Tensor, table: capi.Table, H: int, W: int) -> torch.Ten
     return out
 
 
+def _antiring(y: torch.Tensor, x: torch.Tensor, table: capi.Table, strength: float) -> None:
+    """The anti-ringing clamp in place on y = _forward(x, ...)."""
+    src, out = _planes(x), _planes(y)
+    isz = x.element_size()
+    if src.shape[0]:
+        table.antiring_planes_device(_SAMPLE[x.dtype], strength, src.shape[0], src.data_ptr(), src.stride(1) * isz,
+                                     src.stride(0) * isz, out.data_ptr(), out.stride(1) * isz, out.stride(0) * isz,
+                                     _stream(x.device))
+
+
 class _JincResizeFloat(torch.autograd.Function):
     """float16 / float32 planes: forward resize, backward adjoint (float32, cast to x.dtype)."""
 
@@ -164,9 +181,43 @@ class _JincResizeFloat(torch.autograd.Function):
         return g.view(ctx.src_shape).to(ctx.x_dtype), None, None, None
 
 
+class _JincResizeAntiringFloat(torch.autograd.Function):
+    """float16 / float32 planes with anti-ringing: forward resize + clamp; backward recomputes the resized planes (the
+    resize is deterministic, so they are the forward's bit for bit) and runs the clamp's adjoint (float32, cast to
+    x.dtype).  Only x is kept, so the graph holds what it holds without anti-ringing."""
+
+    @staticmethod
+    def forward(ctx, x, table, width, height, strength):
+        ctx.table, ctx.width, ctx.height, ctx.strength = table, width, height, strength
+        ctx.save_for_backward(x)
+        with torch.cuda.device(x.device):
+            y = _forward(x, table, width, height, 0.0)
+            _antiring(y, x, table, strength)
+        return y
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        (x,) = ctx.saved_tensors
+        with torch.cuda.device(x.device):
+            y = _planes(_forward(x, ctx.table, ctx.width, ctx.height, 0.0))
+            src = _planes(x)
+            g = _planes(grad_out.to(torch.float32))
+            n, h, w = g.shape
+            H, W = src.shape[-2:]
+            g_y = torch.empty((n, h, w), dtype=torch.float32, device=x.device)
+            out = torch.empty((n, H, W), dtype=torch.float32, device=x.device)
+            isz = x.element_size()
+            if n:
+                ctx.table.antiring_adjoint_planes_device(
+                    _SAMPLE[x.dtype], ctx.strength, n, (src.data_ptr(), src.stride(1) * isz, src.stride(0) * isz),
+                    (y.data_ptr(), y.stride(1) * isz, y.stride(0) * isz), (g.data_ptr(), g.stride(1) * 4, g.stride(0) * 4),
+                    (g_y.data_ptr(), w * 4, h * w * 4), (out.data_ptr(), W * 4, H * W * 4), _stream(x.device))
+        return out.view(x.shape).to(x.dtype), None, None, None, None
+
+
 def jinc_resize(x: torch.Tensor, width: int, height: int, *, tap: int = 3, src_left: float = 0.0, src_top: float = 0.0,
                 src_width: float | None = None, src_height: float | None = None, quant_x: int = 256, quant_y: int = 256,
-                blur: float = 0.0, bits: int | None = None) -> torch.Tensor:
+                blur: float = 0.0, bits: int | None = None, antiring: float = 0.0) -> torch.Tensor:
     """Jinc (EWA) resize of every (H, W) plane of the CUDA tensor `x` (..., H, W) to (..., height, width).
 
     dtypes: uint8 (bits 8), uint16 (bits 9..16, default 16; samples are clamped to 2**bits - 1), float16 and float32 (raw
@@ -178,8 +229,12 @@ def jinc_resize(x: torch.Tensor, width: int, height: int, *, tap: int = 3, src_l
     (stride(-2) > width, the leading dimensions packed).  It is a tensor of its own, not a view, so it may be modified in
     place before backward.  float16 / float32 inputs are differentiable with
     respect to x (the adjoint of the resize); the geometry arguments are not.
+
+    antiring (0.0 .. 1.0, default 0 = off) clamps every output sample toward the range of the 2x2 source samples around it,
+    as core.jinc.JincResize's `antiring`; float16 / float32 inputs stay differentiable (DESIGN.md 4.9), the strength is not.
     """
-    bits = _check_args(x, width, height, tap, quant_x, quant_y, bits)
+    bits = _check_args(x, width, height, tap, quant_x, quant_y, bits, antiring)
+    strength = _f32(antiring)
     H, W = x.shape[-2:]
     src_left, src_top = _f32(src_left), _f32(src_top)
     crop_w = _f32(src_width) if src_width is not None else float(W)
@@ -193,9 +248,14 @@ def jinc_resize(x: torch.Tensor, width: int, height: int, *, tap: int = 3, src_l
     with torch.cuda.device(device):
         table = _table(device, key)
     if bits == 0:
-        return _JincResizeFloat.apply(x, table, width, height)
+        if strength == 0.0:
+            return _JincResizeFloat.apply(x, table, width, height)
+        return _JincResizeAntiringFloat.apply(x, table, width, height, strength)
     with torch.cuda.device(device):
-        return _forward(x, table, width, height, float((1 << bits) - 1))
+        y = _forward(x, table, width, height, float((1 << bits) - 1))
+        if strength != 0.0:
+            _antiring(y, x, table, strength)
+        return y
 
 
 __all__ = ["jinc_resize"]

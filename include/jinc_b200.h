@@ -181,6 +181,41 @@ JINC_API int jinc_resize_adjoint_planes_device(jinc_ctx* ctx, const jinc_table* 
 JINC_API int jinc_antiring_plane_device(jinc_ctx* ctx, const jinc_table* t, int sample_bytes, float strength,
                                         const void* d_src, ptrdiff_t src_pitch, void* d_dst, ptrdiff_t dst_pitch,
                                         void* stream);
+/* The clamp above on n_planes planes that jinc_resize_planes_device produced (plane i at d_src + i*src_plane_stride /
+ * d_dst + i*dst_plane_stride, bytes), in place.  Byte-identical to n_planes calls of jinc_antiring_plane_device; one launch
+ * per chunk (records of up to four planes, chunks of at most 65535 records, from the context's ring).  Same sample_bytes,
+ * pitch and alignment rules as jinc_resize_planes_device; strength NaN or outside [0, 1] is JINC_E_INVALID, 0 launches
+ * nothing.  Asynchronous on `stream` (NULL = the context's stream). */
+JINC_API int jinc_antiring_planes_device(jinc_ctx* ctx, const jinc_table* t, int sample_bytes, float strength, int n_planes,
+                                         const void* d_src, ptrdiff_t src_pitch, ptrdiff_t src_plane_stride, void* d_dst,
+                                         ptrdiff_t dst_pitch, ptrdiff_t dst_plane_stride, void* stream);
+/* Gradient of resize + anti-ringing clamp for float32 (sample_bytes 4) and half (JINC_SAMPLE_F16) planes (no reference
+ * counterpart).  d_src: the source planes; d_y: the resized planes as jinc_resize_planes_device stored them, BEFORE the
+ * clamp; d_grad_dst: float32 gradients of the clamped output.  Writes d_grad_y (float32, the output's size: the gradient
+ * reaching the resized planes) and d_grad_src (float32, the source's size).  Per output sample, with y widened to float,
+ * the anchors a0..a3 = src[ay0][ax0], src[ay0][ax1], src[ay1][ax0], src[ay1][ax1] and lo / hi as in
+ * jinc_antiring_plane_device, s the strength and g the output gradient:
+ *   inside (y NaN, or !(y < lo) && !(y > hi); all four anchors NaN included):  g_y = g, nothing routed
+ *   below  (y < lo):  g_y = s == 1 ? +0.0f : __fmul_rn(1 - s, g); the value s == 1 ? g : __fmul_rn(s, g) is routed to the
+ *                     FIRST anchor in a0..a3 order whose widened value == lo (the tie rule: equal anchors, or an anchor
+ *                     that is the same sample twice at the plane's edge, take it in that order)
+ *   above  (y > hi):  the same with hi.
+ * grad_src = A^T g_y + r, A^T exactly jinc_resize_adjoint_planes_device; r[sy][sx] sums the values routed to that sample in
+ * canonical order (output rows ascending, then columns ascending, __fadd_rn starting from the first routed value).  A
+ * sample that receives nothing keeps A^T g_y bit for bit, one that does gets __fadd_rn(A^T g_y, r).  So every bit of the
+ * result is defined independently of kernel, tile, batch position and launch.  These are the derivatives of the
+ * exact-arithmetic piecewise-linear map (at a kink the side given above).  At strength 0 g_y is a copy of g and grad_src
+ * the plain adjoint.  All pointers aligned to their sample size, pitches multiples of it that hold a row and, when
+ * n_planes > 1, plane strides multiples of it that hold a plane; d_grad_src must not overlap d_grad_dst or d_grad_y, nor
+ * d_grad_y d_grad_dst.  JINC_E_INVALID otherwise, for a strength that is NaN or outside [0, 1], or another sample type.
+ * Three launches on `stream` (one copy and the adjoint at strength 0); asynchronous (NULL = the context's stream). */
+JINC_API int jinc_antiring_adjoint_planes_device(jinc_ctx* ctx, const jinc_table* t, int sample_bytes, float strength,
+                                                 int n_planes, const void* d_src, ptrdiff_t src_pitch,
+                                                 ptrdiff_t src_plane_stride, const void* d_y, ptrdiff_t y_pitch,
+                                                 ptrdiff_t y_plane_stride, const float* d_grad_dst, ptrdiff_t g_pitch,
+                                                 ptrdiff_t g_plane_stride, float* d_grad_y, ptrdiff_t gy_pitch,
+                                                 ptrdiff_t gy_plane_stride, float* d_grad_src, ptrdiff_t gs_pitch,
+                                                 ptrdiff_t gs_plane_stride, void* stream);
 /* Introspection of the table's strip plan (no reference counterpart: the reference keeps one weight block per border
  * pixel, src/JincResize.cpp:443-518, and has no notion of patches).  Whole-frame launches of the exact-2x, chunked-cells
  * and integer-ratio kernels run their border strips from descriptors worked out once per table; returns the number of
